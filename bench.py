@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- compaction throughput (MB/s of input bytes) of the B200 engine vs the CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic input: the 8 independent shard
 compactions of BASELINE.json configs[3] -- each one configs[1]'s 8-way merge of 1M-key x 256-byte-doc
@@ -22,6 +22,10 @@ report).  Per-job figures (ms_per_job, stage_ms, roofline) are configs[1]'s.
 --impl reference times the CPU path alone with every host core busy (one full-size shard compaction
 per core, the way dbeel's thread-per-core runtime would run them).
 --workload cfg5 runs BASELINE.json configs[4] instead (dbeel_b200/cfg5.py).
+--dump-outputs DIR writes what the jobs of the last timed step returned (either arm; see dump_job_outputs).  The inputs
+are seeded, so two builds run with the same arguments can be compared file for file.  The GPU arm then gives every job
+its own output buffers (8 x ~2.5 GB more HBM), so its timed kernels write elsewhere than in a run without the flag; the
+JSON line says so under "dump_outputs".  The reference arm dumps the jobs its last step ran, all 8 only when it ran 8.
 """
 from __future__ import annotations
 
@@ -182,6 +186,36 @@ def same_output(a, b) -> bool:
     """(data, index, bloom | None, items) of the engine vs the oracle, byte for byte."""
     return bool(a[3] == b[3] and np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
                 and (a[2] is None) == (b[2] is None) and (a[2] is None or np.array_equal(a[2], b[2])))
+
+
+DUMP_SAMPLE = {"data": 1 << 20, "index": 1 << 18, "bloom": 1 << 18}  # bytes of each output file sampled per job
+DUMP_BLOCK = 1 << 16  # bytes per block sum
+
+
+def dump_job_outputs(out_dir: str, shard_id: int, data, index, bloom, items: int) -> None:
+    """--dump-outputs: one job's output SSTable (uint8 torch tensors on any device, bloom None when there is none) as .npy
+    files that two builds can be compared with, file for file:
+      job<i>_lengths.npy          float64 [.data bytes, .index bytes, .bloom bytes, entries written]
+      job<i>_<file>_sample.npy    float32 bytes of the file at positions drawn from a fixed seed (the whole file if smaller)
+      job<i>_<file>_blocksum.npy  float64 sum of the bytes of every 64 KiB block (exact: a changed byte moves one of them)
+    About 6.6 MB per job of the default workload, 53 MB for its 8 jobs."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    files = {"data": data, "index": index, "bloom": bloom if bloom is not None else torch.zeros(0, dtype=torch.uint8)}
+    np.save(os.path.join(out_dir, f"job{shard_id}_lengths.npy"), np.array([t.numel() for t in files.values()] + [items], np.float64))
+    for k, (name, t) in enumerate(files.items()):
+        n = t.numel()
+        if n <= DUMP_SAMPLE[name]:
+            sample = t
+        else:
+            pos = np.sort(np.random.default_rng([shard_id, k]).integers(0, n, DUMP_SAMPLE[name]))
+            sample = t[torch.from_numpy(pos).to(t.device)]
+        whole = n - n % DUMP_BLOCK
+        sums = t[:whole].view(-1, DUMP_BLOCK).sum(1, dtype=torch.float64)
+        if n > whole:
+            sums = torch.cat([sums, t[whole:].sum(dtype=torch.float64).view(1)])
+        np.save(os.path.join(out_dir, f"job{shard_id}_{name}_sample.npy"), sample.cpu().numpy().astype(np.float32))
+        np.save(os.path.join(out_dir, f"job{shard_id}_{name}_blocksum.npy"), sums.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------ GPU arm
@@ -392,10 +426,12 @@ def run_gpu(args):
     # stream's, so two jobs' stages do not co-run.  Off by default; the rank's jobs run one after the other.
     n_eng = 2 if (len(mine) >= 2 and args.overlap) else 1
     engs = [eng] + [capi.Engine(local) for _ in range(n_eng - 1)]
-    # device-resident inputs of every job of this rank; one output SSTable buffer set per engine, reused job after job
+    # device-resident inputs of every job of this rank; one output SSTable buffer set per engine, reused job after job --
+    # with --dump-outputs one per job, so that every job's output of the last timed step is still there after it
     t_jobs = [[(torch.from_numpy(d).to(dev), torch.from_numpy(i).to(dev)) for d, i in runs] for runs in jobs_runs]
+    slot = list(range(len(mine))) if args.dump_outputs else [j % n_eng for j in range(len(mine))]
     outs = [(torch.empty(dc + 64, dtype=torch.uint8, device=dev), torch.empty(ic + 64, dtype=torch.uint8, device=dev),
-             torch.empty(bc + 64, dtype=torch.uint8, device=dev)) for _ in engs]
+             torch.empty(bc + 64, dtype=torch.uint8, device=dev)) for _ in range(len(mine) if args.dump_outputs else n_eng)]
     d_jobs = [[(d.data_ptr(), d.numel(), i.data_ptr(), i.numel()) for d, i in t_runs] for t_runs in t_jobs]
     d_outs = [(od.data_ptr(), dc, oi.data_ptr(), ic, ob.data_ptr(), bc) for od, oi, ob in outs]
     ext = [torch.cuda.ExternalStream(e_.stream_ptr(), device=dev) for e_ in engs]
@@ -423,11 +459,12 @@ def run_gpu(args):
     # ---- (2) the timed region: K steps, each one pass over this rank's jobs, two in flight when there are two engines
     acc = {"kernel_launches": 0}
     lock = threading.Lock()
+    last = [None] * len(d_jobs)  # (data_len, index_len, bloom_len, items) of every job in the latest step
 
     def worker(ei: int, record: bool):
         n_l = 0
         for j in range(ei, len(d_jobs), n_eng):
-            engs[ei].compact_device(d_jobs[j], d_outs[ei], opts)
+            last[j] = engs[ei].compact_device(d_jobs[j], d_outs[slot[j]], opts)
             if record:
                 n_l += engs[ei].stats()["kernel_launches"]
         if record:
@@ -466,6 +503,11 @@ def run_gpu(args):
     sampler.stop()
     wall_ms = (t1 - t0) * 1e3
     clocks = sampler.summary(t0, t1)
+    if args.dump_outputs:
+        for j, job in enumerate(mine):
+            dl, il, bl, items = last[j]
+            od, oi, ob = outs[slot[j]]
+            dump_job_outputs(args.dump_outputs, job.shard_id, od[:dl], oi[:il], ob[:bl] if bl else None, items)
 
     # max over ranks of the device time (CUDA events on the engines' streams, summed over the K steps)
     tm = torch.tensor([dev_ms, wall_ms], dtype=torch.float64, device=dev)
@@ -618,6 +660,10 @@ def run_gpu(args):
         "parity_all_ranks": parity_all,
         "other_configs": others,
     }
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "jobs_rank0": [j.shard_id for j in mine],
+                                "output_buffers": "one set per job, where a run without --dump-outputs reuses one set per engine: "
+                                                  "the timed kernels wrote to other (and more) HBM than in such a run"}
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -674,11 +720,15 @@ def run_reference(args):
     log(f"[bench ref] {threads} threads x one full cfg2-shaped compaction each ({in_bytes / 1e6:.0f} MB per step), "
         f"{distinct_n} distinct shards generated in {time.time() - t:.0f}s")
 
-    def one(s):
-        oracle.compact(s, False, seed=SEED32, emulate_page_cache=True)
+    kept = {}  # --dump-outputs: shard id -> (data, index, bloom | None, items) of the distinct shards in the last step
 
-    def step():
-        ts = [threading.Thread(target=one, args=(s,)) for s in shards]
+    def one(s, k=0, keep=False):
+        out = oracle.compact(s, False, seed=SEED32, emulate_page_cache=True)
+        if keep and k < distinct_n:
+            kept[k] = out
+
+    def step(keep=False):
+        ts = [threading.Thread(target=one, args=(s, k, keep)) for k, s in enumerate(shards)]
         for th in ts:
             th.start()
         for th in ts:
@@ -704,10 +754,19 @@ def run_reference(args):
     for _ in range(warm):
         step()
     t0 = time.perf_counter()
-    for _ in range(steps):
-        step()
+    for k in range(steps):
+        step(keep=bool(args.dump_outputs) and k == steps - 1)
     dt = time.perf_counter() - t0
     value = in_bytes * steps / 1e6 / dt
+    if args.dump_outputs:
+        import torch
+        for k, (d, i, b, n) in sorted(kept.items()):
+            dump_job_outputs(args.dump_outputs, k, torch.from_numpy(d), torch.from_numpy(i), None if b is None else torch.from_numpy(b), n)
+        dumped = sorted(kept)
+        kept.clear()
+        if len(dumped) < N_JOBS:
+            log(f"[bench ref] --dump-outputs: wrote jobs {dumped} only, not all {N_JOBS}: the last step ran {threads} concurrent "
+                f"jobs over {distinct_n} distinct shards")
     # secondary: one thread alone on the same shape (no memory-bandwidth sharing)
     t1 = time.perf_counter()
     one(shards[0])
@@ -723,6 +782,8 @@ def run_reference(args):
             "config": cfg_line, "threads": threads, "jobs_per_step": threads, "one_thread_alone_mbs": round(alone, 1),
             "cpu_baseline": {"value": round(value, 2), "unit": UNIT, "cores": threads, "kind": "port", "sample": sample},
             "e2e": {"value": round(value, 2), "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "jobs": dumped}
     print(json.dumps(line), flush=True)
 
 
@@ -738,7 +799,14 @@ def main():
     ap.add_argument("--workload", default="cfg2", choices=["cfg2", "cfg3", "cfg5"],
                     help="cfg2 (default): BASELINE.json's headline, 8 shard jobs of configs[1]'s shape; cfg5: configs[4]")
     ap.add_argument("--writes", type=int, default=0, help="cfg5: arrivals in the stream (default 32M)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what every job of the last step returned (length, seeded byte samples "
+                         "and block sums of its .data / .index / .bloom) as DIR/job<i>_*.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload == "cfg5":
+        ap.error("--dump-outputs covers the compaction jobs of the cfg2 / cfg3 workloads, not cfg5")
     if args.impl == "reference":
         run_reference(args)
     else:
