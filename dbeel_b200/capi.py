@@ -30,6 +30,10 @@ FLAG_VERIFY_SORTED = 0x1
 FLAG_REFERENCE_READER = 0x2  # decode runs like read_next_entry (lsm_tree.rs:1158-1170): offset / key_size ignored, timestamps range-checked
 DEFAULT_BLOOM_MIN_SIZE = 1_048_576
 DEFAULT_BLOOM_FP = 0.01
+SCAN_REFERENCE = 0  # between_cmp read literally (migration.rs:54-60): a wrapped range holds for every hash
+SCAN_EXACT = 1      # a wrapped range (end < start) is [start, 2^32) u [0, end)
+MAX_SCAN_RANGES = 256
+SCAN_END, SCAN_DECODE, SCAN_READ = 0, 1, 2  # dbeel_scan_stop.reason
 
 EXPORTS = ["dbeel_abi_version", "dbeel_engine_create", "dbeel_engine_destroy", "dbeel_compact_bound",
            "dbeel_compact", "dbeel_compact_stream", "dbeel_compact_device", "dbeel_compact_submit", "dbeel_poll", "dbeel_wait",
@@ -39,7 +43,8 @@ EXPORTS = ["dbeel_abi_version", "dbeel_engine_create", "dbeel_engine_destroy", "
            "dbeel_bloom_bitmap_bytes", "dbeel_bloom_k_num", "dbeel_bloom_file_size", "dbeel_host_alloc",
            "dbeel_host_free", "dbeel_last_stats", "dbeel_last_error", "dbeel_strerror",
            "dbeel_murmur3_32", "dbeel_ring_owner", "dbeel_shard_ring", "dbeel_route_device", "dbeel_flush_many_sparse_device",
-           "dbeel_gpu_numa_node", "dbeel_bind_to_gpu", "dbeel_memtable_cuts_device", "dbeel_engine_stream"]
+           "dbeel_gpu_numa_node", "dbeel_bind_to_gpu", "dbeel_memtable_cuts_device", "dbeel_engine_stream",
+           "dbeel_scan_ranges", "dbeel_scan_ranges_device"]
 
 
 class Run(C.Structure):
@@ -78,6 +83,14 @@ class JobResult(C.Structure):
 class Table(C.Structure):
     _fields_ = [("data", C.c_void_p), ("data_len", C.c_uint64), ("index", C.c_void_p), ("index_len", C.c_uint64),
                 ("bloom", C.c_void_p), ("bloom_len", C.c_uint64)]
+
+
+class HashRange(C.Structure):
+    _fields_ = [("start", C.c_uint32), ("end", C.c_uint32)]
+
+
+class ScanStop(C.Structure):
+    _fields_ = [("table", C.c_int32), ("reason", C.c_uint32), ("record", C.c_uint64)]
 
 
 class LookupResult(C.Structure):
@@ -216,6 +229,11 @@ def lib():
         L.dbeel_flush_many_sparse_device.restype = C.c_int
         L.dbeel_flush_many_sparse_device.argtypes = [C.c_void_p, C.POINTER(Run), C.c_uint32, C.c_uint64, C.POINTER(Out),
                                                      C.POINTER(FlushTable)]
+        for name in ("dbeel_scan_ranges", "dbeel_scan_ranges_device"):
+            f = getattr(L, name)
+            f.restype = C.c_int
+            f.argtypes = [C.c_void_p, C.POINTER(Run), C.c_uint32, C.POINTER(HashRange), C.c_uint32, C.c_uint32, C.POINTER(Out),
+                          C.POINTER(FlushTable), C.POINTER(ScanStop)]
         _lib = L
     return _lib
 
@@ -567,6 +585,53 @@ class Engine:
             arr[j] = Table(t[0], t[1], t[2], t[3], t[4] if t[5] else None, t[5])
         self._check(lib().dbeel_get_many_device(self._h, arr, len(tables), keys_ptr, offsets_ptr, n_keys, mode,
                                                 results_ptr), "dbeel_get_many_device")
+
+    # ---- hash-range scans (shard migration) ----------------------------------------------
+    @staticmethod
+    def _scan_args(ranges):
+        rng = (HashRange * max(1, len(ranges)))()
+        for j, (a, b) in enumerate(ranges):
+            rng[j] = HashRange(a, b)
+        return rng, (FlushTable * max(1, len(ranges)))(), ScanStop()
+
+    @staticmethod
+    def _scan_result(per_range, n, stop):
+        rows = [{k: int(getattr(t, k)) for k, _ in FlushTable._fields_} for t in per_range[:n]]
+        return rows, (int(stop.table), int(stop.reason), int(stop.record))
+
+    def scan_ranges(self, tables: Sequence[Tuple[object, object]], ranges: Sequence[Tuple[int, int]],
+                    mode: int = SCAN_REFERENCE, caps: Optional[Tuple[int, int]] = None):
+        """dbeel_scan_ranges over host buffers.  tables: (data, index) in iteration order (SSTables oldest first, then
+        the memtables as sorted runs); ranges: (start, end) hash ranges.  Returns (data, index, per_range, stop):
+        per_range rows carry the dbeel_flush_table fields, stop = (table | -1, reason, record).  caps: (data_cap,
+        index_cap), default the bound that always suffices."""
+        keep = [(_u8(d), _u8(i)) for d, i in tables]
+        arr = (Run * max(1, len(keep)))()
+        for j, (d, i) in enumerate(keep):
+            arr[j] = Run(d.ctypes.data, d.size, i.ctypes.data, i.size)
+        dc, ic = caps if caps is not None else (sum(d.size for d, _ in keep), 16 * sum(i.size // 16 for _, i in keep))
+        od, oi = np.empty(max(1, dc), np.uint8), np.empty(max(1, ic), np.uint8)
+        out = Out(od.ctypes.data, dc, 0, oi.ctypes.data, ic, 0, None, 0, 0, 0)
+        rng, per_range, stop = self._scan_args(ranges)
+        self._check(lib().dbeel_scan_ranges(self._h, arr, len(keep), rng, len(ranges), mode, C.byref(out), per_range,
+                                            C.byref(stop)), "dbeel_scan_ranges")
+        rows, st = self._scan_result(per_range, len(ranges), stop)
+        return od[:out.data_len], oi[:out.index_len], rows, st
+
+    def scan_ranges_device(self, tables: Sequence[Tuple[int, int, int, int]], ranges: Sequence[Tuple[int, int]],
+                           out_ptrs: Tuple[int, int, int, int], mode: int = SCAN_REFERENCE):
+        """dbeel_scan_ranges_device: tables (data_ptr, data_len, index_ptr, index_len) and out_ptrs (data_ptr, data_cap,
+        index_ptr, index_cap) in device memory.  Returns (data_len, index_len, per_range, stop)."""
+        arr = (Run * max(1, len(tables)))()
+        for j, (dp, dl, ip, il) in enumerate(tables):
+            arr[j] = Run(dp, dl, ip, il)
+        dp, dc, ip, ic = out_ptrs
+        out = Out(dp, dc, 0, ip, ic, 0, None, 0, 0, 0)
+        rng, per_range, stop = self._scan_args(ranges)
+        self._check(lib().dbeel_scan_ranges_device(self._h, arr, len(tables), rng, len(ranges), mode, C.byref(out),
+                                                   per_range, C.byref(stop)), "dbeel_scan_ranges_device")
+        rows, st = self._scan_result(per_range, len(ranges), stop)
+        return int(out.data_len), int(out.index_len), rows, st
 
     # ---- device buffers (raw pointers; torch tensors own the memory) -------------------
     def compact_device(self, runs: Sequence[Tuple[int, int, int, int]], out_ptrs: Tuple[int, int, int, int, int, int],

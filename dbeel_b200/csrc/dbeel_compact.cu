@@ -26,6 +26,7 @@
 #include "gather_fb.cuh"
 #include "lookup.cuh"
 #include "route.cuh"
+#include "scan.cuh"
 #include "wal.cuh"
 #include "host/stream_pump.h"
 
@@ -1484,11 +1485,12 @@ int route_entry(dbeel_engine *e, const dbeel_run *batch, const uint32_t *ring, u
     p.out_index = static_cast<uint4 *>(out_index);
     p.hash64 = out_hash64 ? reinterpret_cast<unsigned long long *>(e->route_ws + o_h64) : nullptr;
     p.out_hash64 = static_cast<unsigned long long *>(out_hash64);
+    p.stop = nullptr;
     CU(cudaEventRecord(e->ev[EV_START], s));
     k_copy_words<<<(n_shards + 255) / 256, 256, 0, s>>>(reinterpret_cast<uint32_t *>(e->route_ws + o_ring), reinterpret_cast<const uint32_t *>(e->pin_dev), n_shards);
     CU(cudaMemsetAsync(p.totals, 0, 8ull * 3 * n_shards, s));
     CU(cudaMemsetAsync(p.totals + 3 * n_shards, 0xFF, 8, s));
-    k_route_hash<<<p.n_blocks, kRouteThreads, 0, s>>>(p);
+    k_route_hash<false><<<p.n_blocks, kRouteThreads, 0, s>>>(p);
     k_route_scan<<<n_shards, 1024, 0, s>>>(p);
     unsigned long long *host_tot = reinterpret_cast<unsigned long long *>(e->pin + 4096);
     k_route_starts<<<1, 256, 0, s>>>(p, reinterpret_cast<unsigned long long *>(e->pin_dev + 4096));
@@ -1842,6 +1844,248 @@ int compact_many_entry(dbeel_engine *e, const dbeel_job *jobs, uint32_t n_jobs, 
     return DBEEL_OK;
 }
 
+// ------------------------------------------------------------------------------------ hash-range scans (scan.cuh)
+
+// The device-resident scan.  tables / out hold device pointers; ranges, per_range and stop live in the host's memory.
+// data_bound / index_bound: what the selected entries can take at most (the scanned tables' .data bytes, 16 per record);
+// the caller's caps above them change nothing.
+int run_scan_device(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges, uint32_t n_ranges,
+                    uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range, dbeel_scan_stop *stop) {
+    dbeel_stats &st = e->stats;
+    // the scan ends in front of the first table without a record: its first 16-byte index read hits EOF (lsm_tree.rs:250)
+    uint32_t nt = 0;
+    uint64_t n64 = 0, data_bound = 0, in_bytes = 0;
+    while (nt < n_tables && tables[nt].index_len >= DBEEL_INDEX_ENTRY_SIZE) {
+        n64 += tables[nt].index_len / DBEEL_INDEX_ENTRY_SIZE;
+        data_bound += tables[nt].data_len;
+        in_bytes += tables[nt].data_len + tables[nt].index_len;
+        nt++;
+    }
+    const bool empty_stop = nt < n_tables;
+    if (n64 >= 0xFFFFFFF0ull) return fail(e, DBEEL_ERR_TOO_MANY_ENTRIES, "more than 2^32 - 16 records in one scan");
+    const uint32_t N = (uint32_t)n64;
+    st.entries_in = N;
+    st.input_bytes = in_bytes;
+    *stop = empty_stop ? dbeel_scan_stop{(int32_t)nt, DBEEL_SCAN_READ, 0} : dbeel_scan_stop{-1, DBEEL_SCAN_END, 0};
+    if (N == 0) return DBEEL_OK;
+
+    // no ranges: one class that selects nothing, so the scan still finds its stop
+    const uint32_t n_cls = n_ranges ? n_ranges : 1;
+    const uint64_t data_cap = std::min<uint64_t>(out->data_cap, data_bound), index_cap = std::min<uint64_t>(out->index_cap, 16ull * N);
+    const uint64_t gather_tiles = (data_cap + kGatherTileBytes - 1) / kGatherTileBytes;
+    const uint32_t n_blocks = (N + kRouteThreads - 1) / kRouteThreads;
+    const uint64_t res_tiles = (N + kResolveThreads - 1) / kResolveThreads, res_chunks = (res_tiles + 1023) / 1024;
+
+    uint64_t off = 0;
+    auto carve = [&](uint64_t b) { uint64_t o2 = off; off = align_up(off + b, kAlign); return o2; };
+    // header block (host-initialised, goes down through the mapped pinned block): ctl | tables | ranges | mem_table, stop
+    const uint64_t o_ctl = carve(sizeof(Ctl)), o_tab = carve(sizeof(ScanTable) * nt), o_rng = carve(8ull * n_cls);
+    const uint64_t o_mt = carve(16ull * (n_cls + 1) + 8); // k_flush_table's rows, then the stop key: published together
+    const uint64_t header_bytes = off;
+    const uint64_t o_seg = carve(sizeof(Seg) * n_cls), o_tot = carve(8ull * (3 * n_cls + 1)), o_hist = carve(4ull * n_blocks * n_cls);
+    const uint64_t o_cls = carve(4ull * N), o_rec = carve(16ull * N), o_res = carve(16ull * N), o_src = carve(8ull * N);
+    const uint64_t o_tb = carve(8 * res_tiles), o_tc = carve(4 * res_tiles), o_cb = carve(8 * res_chunks), o_cc = carve(4 * res_chunks);
+    const uint64_t o_tf = carve(4ull * (gather_tiles + 2));
+    int rc = ensure_device(e, &e->ws, &e->ws_cap, off);
+    const uint64_t o_hctl = header_bytes, o_hmt = o_hctl + align_up(sizeof(Ctl), 64), o_htot = o_hmt + align_up(16ull * (n_cls + 1) + 8, 64);
+    if (!rc) rc = ensure_pinned(e, o_htot + 8ull * (3 * n_cls + 1));
+    if (rc) return rc;
+    uint8_t *ws = e->ws, *h = e->pin;
+
+    memset(h, 0, header_bytes);
+    ScanTable *ht = reinterpret_cast<ScanTable *>(h + o_tab);
+    for (uint32_t t = 0, base = 0; t < nt; t++) {
+        ht[t] = ScanTable{static_cast<const uint8_t *>(tables[t].data), tables[t].data_len, static_cast<const uint4 *>(tables[t].index), base,
+                          (uint32_t)(tables[t].index_len / DBEEL_INDEX_ENTRY_SIZE)};
+        base += ht[t].n;
+    }
+    uint2 *hr = reinterpret_cast<uint2 *>(h + o_rng);
+    for (uint32_t r = 0; r < n_ranges; r++) hr[r] = make_uint2(ranges[r].start, ranges[r].end);
+    if (!n_ranges) hr[0] = make_uint2(0, 0); // start == end holds for no hash in either mode
+    unsigned long long *hstop = reinterpret_cast<unsigned long long *>(h + o_mt + 16ull * (n_cls + 1));
+    *hstop = empty_stop ? (((unsigned long long)N << 2) | DBEEL_SCAN_READ) : ~0ull;
+
+    ScanParams sp;
+    sp.tables = reinterpret_cast<const ScanTable *>(ws + o_tab);
+    sp.n_tables = nt;
+    sp.n = N;
+    sp.ranges = reinterpret_cast<const uint2 *>(ws + o_rng);
+    sp.n_ranges = n_cls;
+    sp.mode = mode;
+    sp.cls = reinterpret_cast<uint32_t *>(ws + o_cls);
+    sp.rec = reinterpret_cast<uint4 *>(ws + o_rec);
+    sp.stop = reinterpret_cast<unsigned long long *>(ws + o_mt + 16ull * (n_cls + 1));
+    sp.totals = reinterpret_cast<unsigned long long *>(ws + o_tot);
+    sp.ctl = reinterpret_cast<Ctl *>(ws + o_ctl);
+    sp.seg = reinterpret_cast<Seg *>(ws + o_seg);
+    sp.data_cap = data_cap;
+    sp.index_cap = index_cap;
+
+    RouteParams rp;
+    memset(&rp, 0, sizeof rp);
+    rp.index = sp.rec; // the res record of every selected entry is what the split moves
+    rp.n = N;
+    rp.n_shards = n_cls;
+    rp.n_blocks = n_blocks;
+    rp.shard_of = sp.cls;
+    rp.hist = reinterpret_cast<uint32_t *>(ws + o_hist);
+    rp.totals = sp.totals;
+    rp.out_index = reinterpret_cast<uint4 *>(ws + o_res);
+    rp.stop = sp.stop;
+
+    Params p;
+    memset(&p, 0, sizeof p);
+    p.n_total = N;
+    p.ctl = sp.ctl;
+    p.seg[0] = sp.seg; // n_levels 0: a range is a group, its first res position its segment start
+    p.n_groups = n_cls;
+    p.mem_table = reinterpret_cast<unsigned long long *>(ws + o_mt);
+    p.tile_bytes = reinterpret_cast<unsigned long long *>(ws + o_tb);
+    p.tile_count = reinterpret_cast<uint32_t *>(ws + o_tc);
+    p.chunk_bytes = reinterpret_cast<unsigned long long *>(ws + o_cb);
+    p.chunk_count = reinterpret_cast<uint32_t *>(ws + o_cc);
+    p.src_ptr = reinterpret_cast<unsigned long long *>(ws + o_src);
+    p.tile_first = reinterpret_cast<uint32_t *>(ws + o_tf);
+    p.tile_first_n = (uint32_t)(gather_tiles + 2);
+    p.out_data = static_cast<uint8_t *>(out->data);
+    p.out_index = static_cast<uint4 *>(out->index);
+    const uint4 *res = rp.out_index;
+
+    cudaStream_t s = e->stream;
+    uint32_t launches = 0;
+    CU(cudaEventRecord(e->ev[EV_START], s));
+    k_copy_words<<<(uint32_t)((header_bytes / 4 + 255) / 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(ws), reinterpret_cast<const uint32_t *>(e->pin_dev),
+                                                                            (uint32_t)(header_bytes / 4));
+    CU(cudaMemsetAsync(sp.totals, 0, 8ull * (3 * n_cls + 1), s));
+    k_scan_classify<<<(N + 255) / 256, 256, 0, s>>>(sp);
+    CU(cudaEventRecord(e->ev[EV_EXTRACT], s));
+    k_route_hash<true><<<n_blocks, kRouteThreads, 0, s>>>(rp);
+    k_route_scan<<<n_cls, 1024, 0, s>>>(rp);
+    k_route_starts<<<1, 256, 0, s>>>(rp, reinterpret_cast<unsigned long long *>(e->pin_dev + o_htot));
+    k_route_scatter<<<n_blocks, kRouteThreads, 0, s>>>(rp);
+    k_scan_plan<<<1, 256, 0, s>>>(sp);
+    k_scan_res_tiles<<<(uint32_t)res_tiles, kResolveThreads, 0, s>>>(p, res);
+    k_scan_tiles<<<(uint32_t)res_chunks, 1024, 0, s>>>(p);
+    k_scan_chunks<<<1, 1024, 0, s>>>(p);
+    k_emit<<<(uint32_t)res_tiles, kResolveThreads, 0, s>>>(p, res);
+    k_flush_table<<<(n_cls + 1 + 127) / 128, 128, 0, s>>>(p, res);
+    CU(cudaEventRecord(e->ev[EV_RESOLVE], s));
+    launches += 12;
+    if (gather_tiles) {
+        if (((uintptr_t)out->data & 31) == 0) k_gather32<false, false, false, true><<<(uint32_t)gather_tiles, kGatherThreads, 0, s>>>(p);
+        else k_gather<<<(uint32_t)gather_tiles, kGatherThreads, 0, s>>>(p);
+        launches++;
+    }
+    k_rebase_index<<<(N + 255) / 256, 256, 0, s>>>(p); // after the gather: it reads the offsets as stream offsets
+    CU(cudaEventRecord(e->ev[EV_GATHER], s));
+    k_publish<<<1, 256, 0, s>>>(reinterpret_cast<uint32_t *>(e->pin_dev + o_hctl), reinterpret_cast<const uint32_t *>(sp.ctl),
+                                (uint32_t)(sizeof(Ctl) / 4), reinterpret_cast<uint32_t *>(e->pin_dev + o_hmt),
+                                reinterpret_cast<const uint32_t *>(p.mem_table), (uint32_t)(4 * (n_cls + 1) + 2));
+    launches += 2;
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(s));
+
+    const Ctl *hc = reinterpret_cast<const Ctl *>(h + o_hctl);
+    const unsigned long long *hmt = reinterpret_cast<const unsigned long long *>(h + o_hmt);
+    const unsigned long long key = hmt[2 * (n_cls + 1)];
+    st.kernel_launches = launches;
+    cudaEventElapsedTime(&st.ms_total, e->ev[EV_START], e->ev[EV_GATHER]);
+    cudaEventElapsedTime(&st.ms_extract, e->ev[EV_START], e->ev[EV_EXTRACT]);
+    cudaEventElapsedTime(&st.ms_resolve, e->ev[EV_EXTRACT], e->ev[EV_RESOLVE]);
+    cudaEventElapsedTime(&st.ms_gather, e->ev[EV_RESOLVE], e->ev[EV_GATHER]);
+    st.entries_valid = key == ~0ull ? N : (uint32_t)(key >> 2);
+    if (key != ~0ull && !(empty_stop && (key >> 2) == N)) {
+        const uint32_t o = (uint32_t)(key >> 2);
+        uint32_t t = 0;
+        while (t + 1 < nt && ht[t + 1].base <= o) t++;
+        *stop = dbeel_scan_stop{(int32_t)t, (uint32_t)(key & 3), (uint64_t)(o - ht[t].base)};
+    }
+    if (hc->flags & kScanOverCap) return fail(e, DBEEL_ERR_CAPACITY, "scan output larger than the output buffers");
+    out->data_len = hc->out_data_len;
+    out->items_written = hc->out_items;
+    out->index_len = 16ull * hc->out_items;
+    for (uint32_t r = 0; r < n_ranges; r++) {
+        dbeel_flush_table &row = per_range[r];
+        row.data_off = hmt[2 * r];
+        row.data_len = hmt[2 * (r + 1)] - hmt[2 * r];
+        row.items = hmt[2 * (r + 1) + 1] - hmt[2 * r + 1];
+        row.index_off = hmt[2 * r + 1] * 16;
+        row.index_len = row.items * 16;
+    }
+    st.entries_out = hc->out_items;
+    st.output_bytes = out->data_len + out->index_len;
+    st.gather_bytes = 2 * out->data_len + out->index_len + 8ull * hc->out_items;
+    st.partitions = 1;
+    return DBEEL_OK;
+}
+
+int scan_entry(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges, uint32_t n_ranges,
+               uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range, dbeel_scan_stop *stop, bool device) {
+    if (!e) return DBEEL_ERR_INVALID_ARG;
+    if (!out || !stop || (n_tables && !tables) || (n_ranges && (!ranges || !per_range))) return fail(e, DBEEL_ERR_INVALID_ARG, "null argument");
+    if (mode > DBEEL_SCAN_EXACT) return fail(e, DBEEL_ERR_INVALID_ARG, "unknown scan mode");
+    if (n_ranges > DBEEL_MAX_SCAN_RANGES) return fail(e, DBEEL_ERR_INVALID_ARG, "more than DBEEL_MAX_SCAN_RANGES ranges");
+    for (uint32_t t = 0; t < n_tables; t++) {
+        if ((tables[t].data_len && !tables[t].data) || (tables[t].index_len >= 16 && !tables[t].index)) return fail(e, DBEEL_ERR_INVALID_ARG, "null table buffer");
+        if (device && ((uintptr_t)tables[t].index & 15)) return fail(e, DBEEL_ERR_INVALID_ARG, "device .index buffers must be 16-byte aligned");
+    }
+    if (device && (((uintptr_t)out->data | (uintptr_t)out->index) & 15)) return fail(e, DBEEL_ERR_INVALID_ARG, "device output buffers must be 16-byte aligned");
+    if (e->busy) return fail(e, DBEEL_ERR_BUSY, "engine busy");
+    BusyGuard g(e);
+    e->err.clear();
+    e->stats = dbeel_stats{};
+    out->data_len = out->index_len = out->bloom_len = out->items_written = 0;
+    for (uint32_t r = 0; r < n_ranges; r++) per_range[r] = dbeel_flush_table{0, 0, 0, 0, 0};
+    *stop = dbeel_scan_stop{-1, DBEEL_SCAN_END, 0};
+    cudaError_t ce = cudaSetDevice(e->device);
+    if (ce != cudaSuccess) return fail(e, DBEEL_ERR_CUDA, "cudaSetDevice", ce);
+    if (device) {
+        if ((out->data_cap && !out->data) || (out->index_cap && !out->index)) return fail(e, DBEEL_ERR_INVALID_ARG, "null output buffer");
+        return run_scan_device(e, tables, n_tables, ranges, n_ranges, mode, out, per_range, stop);
+    }
+    // host buffers: every table goes down whole, the outputs come back (the tree must fit in device memory)
+    uint64_t need = 0, data_bound = 0, n_rec = 0;
+    for (uint32_t t = 0; t < n_tables; t++) {
+        need += align_up(tables[t].data_len + 16, kAlign) + align_up(tables[t].index_len + 16, kAlign);
+        data_bound += tables[t].data_len;
+        n_rec += tables[t].index_len / DBEEL_INDEX_ENTRY_SIZE;
+    }
+    if ((out->data_cap && !out->data) || (out->index_cap && !out->index)) return fail(e, DBEEL_ERR_INVALID_ARG, "null output buffer");
+    const uint64_t dcap = std::min<uint64_t>(out->data_cap, data_bound), icap = std::min<uint64_t>(out->index_cap, 16 * n_rec);
+    int rc = ensure_device(e, &e->stage_in, &e->stage_in_cap, std::max<uint64_t>(need, 256));
+    if (!rc) rc = ensure_device(e, &e->stage_out, &e->stage_out_cap, align_up(dcap + 16, kAlign) + icap + 16);
+    if (rc) return rc;
+    cudaStream_t s = e->stream;
+    CU(cudaEventRecord(e->ev[EV_H2D0], s));
+    std::vector<dbeel_run> dt(n_tables);
+    uint64_t pos = 0;
+    for (uint32_t t = 0; t < n_tables; t++) {
+        uint8_t *dd = e->stage_in + pos;
+        pos += align_up(tables[t].data_len + 16, kAlign);
+        uint8_t *di = e->stage_in + pos;
+        pos += align_up(tables[t].index_len + 16, kAlign);
+        if (tables[t].data_len) CU(cudaMemcpyAsync(dd, tables[t].data, tables[t].data_len, cudaMemcpyHostToDevice, s));
+        if (tables[t].index_len) CU(cudaMemcpyAsync(di, tables[t].index, tables[t].index_len, cudaMemcpyHostToDevice, s));
+        dt[t] = dbeel_run{dd, tables[t].data_len, di, tables[t].index_len};
+    }
+    CU(cudaEventRecord(e->ev[EV_H2D1], s));
+    dbeel_out dout = {e->stage_out, dcap, 0, e->stage_out + align_up(dcap + 16, kAlign), icap, 0, nullptr, 0, 0, 0};
+    rc = run_scan_device(e, dt.data(), n_tables, ranges, n_ranges, mode, &dout, per_range, stop);
+    CU(cudaEventSynchronize(e->ev[EV_H2D1]));
+    cudaEventElapsedTime(&e->stats.ms_h2d, e->ev[EV_H2D0], e->ev[EV_H2D1]);
+    if (rc) return rc;
+    CU(cudaEventRecord(e->ev[EV_D2H0], s));
+    if (dout.data_len) CU(cudaMemcpyAsync(out->data, dout.data, dout.data_len, cudaMemcpyDeviceToHost, s));
+    if (dout.index_len) CU(cudaMemcpyAsync(out->index, dout.index, dout.index_len, cudaMemcpyDeviceToHost, s));
+    CU(cudaEventRecord(e->ev[EV_D2H1], s));
+    CU(cudaStreamSynchronize(s));
+    cudaEventElapsedTime(&e->stats.ms_d2h, e->ev[EV_D2H0], e->ev[EV_D2H1]);
+    out->data_len = dout.data_len;
+    out->index_len = dout.index_len;
+    out->items_written = dout.items_written;
+    return DBEEL_OK;
+}
+
 } // namespace
 
 // ------------------------------------------------------------------------------------ C ABI
@@ -2184,6 +2428,18 @@ int dbeel_wal_flush(dbeel_engine *e, const void *wal, uint64_t wal_len, uint32_t
 int dbeel_wal_flush_device(dbeel_engine *e, const void *wal, uint64_t wal_len, uint32_t capacity, dbeel_out *out) {
     REFUSE_WHILE_ASYNC(e);
     return wal_flush_entry(e, wal, wal_len, capacity, out, true);
+}
+
+int dbeel_scan_ranges(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges, uint32_t n_ranges,
+                      uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range, dbeel_scan_stop *stop) {
+    REFUSE_WHILE_ASYNC(e);
+    return scan_entry(e, tables, n_tables, ranges, n_ranges, mode, out, per_range, stop, false);
+}
+
+int dbeel_scan_ranges_device(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges,
+                             uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range, dbeel_scan_stop *stop) {
+    REFUSE_WHILE_ASYNC(e);
+    return scan_entry(e, tables, n_tables, ranges, n_ranges, mode, out, per_range, stop, true);
 }
 
 void *dbeel_host_alloc(uint64_t bytes) {

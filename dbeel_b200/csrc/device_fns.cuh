@@ -345,4 +345,31 @@ DB_HD uint32_t ring_owner(uint32_t n_shards, uint32_t key_hash, LoadRing ring) {
     return lo == n_shards ? 0u : lo;
 }
 
+// ------------------------------------------------------------------------------------
+// Hash-range scans (the iterator behind shard migration: migrate_actions, src/tasks/migration.rs:62-131, over
+// LSMTree::iter_filter, src/storage_engine/lsm_tree.rs:133-282).
+
+// between_cmp (migration.rs:54-60).  Scan mode 0 (DBEEL_SCAN_REFERENCE) is the literal predicate: a wrapped range
+// (end < start) holds for every hash, start == end for none.  Mode 1 (DBEEL_SCAN_EXACT) reads a wrapped range as
+// [start, 2^32) u [0, end).
+DB_HD bool hash_in_range(uint32_t hash, uint32_t start, uint32_t end, uint32_t mode) {
+    if (end < start) return mode ? (hash >= start || hash < end) : (hash < start || hash >= end);
+    return start <= hash && hash < end;
+}
+
+// AsyncIter::read_one's read of one entry (lsm_tree.rs:250-262): read_at(offset, full_size) on the .data file.  The
+// reference asserts full_size != 0 (cached_file_reader.rs:82) and panics on bytes past the end of the file; both stop a
+// scan.  data_len is the .data file's length.
+DB_HD bool entry_readable(uint64_t offset, uint32_t full_size, uint64_t data_len) {
+    return full_size != 0 && offset <= data_len && (uint64_t)full_size <= data_len - offset;
+}
+
+// bincode Entry of EXACTLY full_size bytes (reject_trailing_bytes, utils/bincode.rs): klen:u64 | key | dlen:u64 | data |
+// ts:i128, i.e. 8 + klen + 8 + dlen + 16 == full_size.  entry_key_fits is the part that depends on klen alone (dlen lies
+// behind the key); entry_decodes is the whole rule, timestamp range included (utils/timestamp_nanos.rs).
+DB_HD bool entry_key_fits(uint64_t full_size, uint64_t klen) { return full_size >= 32 && klen <= full_size - 32; }
+DB_HD bool entry_decodes(uint64_t full_size, uint64_t klen, uint64_t dlen, uint64_t ts_lo, uint64_t ts_hi) {
+    return entry_key_fits(full_size, klen) && dlen == full_size - 32 - klen && ts_decodes(ts_lo, ts_hi);
+}
+
 } // namespace dbeel

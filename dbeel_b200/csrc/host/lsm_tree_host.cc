@@ -631,6 +631,35 @@ int dbeel_tree_get_many(dbeel_tree *t, const void *keys, const uint64_t *key_off
     return rc;
 }
 
+int dbeel_tree_scan_ranges(dbeel_tree *t, const dbeel_run *memtables, uint32_t n_memtables, const dbeel_hash_range *ranges,
+                           uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range, dbeel_scan_stop *stop) {
+    if (!t || (n_memtables && !memtables) || !stop) return DBEEL_ERR_INVALID_ARG;
+    t->err.clear();
+    // AsyncIter walks `self.sstables` (ascending index) and then the memtables (lsm_tree.rs:155-173, 213-282); an empty
+    // memtable yields nothing and is left out (an empty table in front of the engine stops the scan)
+    const size_t n = t->sstables.size();
+    std::vector<PinnedBuf> data(n), index(n);
+    std::vector<dbeel_run> tables;
+    std::vector<int32_t> position; // tables[k] is the caller's table position[k]: SSTables, then memtables
+    for (size_t i = 0; i < n; i++) {
+        const uint64_t idx = t->sstables[i].index;
+        int rc = read_file(t, file_path(t->dir, idx, kData), &data[i]);
+        if (!rc) rc = read_file(t, file_path(t->dir, idx, kIndex), &index[i]);
+        if (rc) return rc;
+        tables.push_back(dbeel_run{data[i].p, data[i].len, index[i].p, index[i].len});
+        position.push_back((int32_t)i);
+    }
+    for (uint32_t m = 0; m < n_memtables; m++) {
+        if (memtables[m].index_len < DBEEL_INDEX_ENTRY_SIZE) continue;
+        tables.push_back(memtables[m]);
+        position.push_back((int32_t)(n + m));
+    }
+    int rc = dbeel_scan_ranges(t->engine, tables.data(), (uint32_t)tables.size(), ranges, n_ranges, mode, out, per_range, stop);
+    if (stop->table >= 0 && (size_t)stop->table < position.size()) stop->table = position[stop->table];
+    if (rc) t->err = dbeel_last_error(t->engine);
+    return rc;
+}
+
 int dbeel_tree_recover_wal(dbeel_tree *t, uint32_t tree_capacity, uint64_t *wal_file_index, uint64_t *items_written) {
     if (!t) return DBEEL_ERR_INVALID_ARG;
     t->err.clear();

@@ -9,9 +9,12 @@
 // arrival batch with SPARSE offsets: dbeel_flush_many_sparse_device flushes it without copying a payload byte twice.
 //
 //   k_route_hash     per arrival: validate the frame, murmur3_32(key), owner; per-block histogram of owners
+//                    (kClassIn: the owner -- any per-entry class id -- is already in shard_of; the hash-range scan,
+//                    scan.cuh, classifies there and drops every entry at or after its stop ordinal here)
 //   k_route_scan     one CTA per shard: exclusive scan of that shard's column over the blocks
 //   k_route_starts   one warp: shard start positions (counts, bytes) -> pinned host block
 //   k_route_scatter  per arrival: stable position = shard start + blocks before + warps before + lanes before
+//                    (it moves whatever 16-byte record `index` holds: the scan hands it res records, kernels.cuh K4)
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -38,10 +41,12 @@ struct RouteParams {
     uint4 *out_index;                 // [n] routed records, shard-major
     unsigned long long *hash64;       // [n] arrival order: (murmur3_32(key, kCutSeed) << 32) | murmur3_32(key, 0), or null
     unsigned long long *out_hash64;   // [n] the same, shard-major (input of k_memtable_cuts)
+    const unsigned long long *stop;   // k_route_hash<true>: (stop ordinal << 2) | reason -- entries at or after it count nowhere
 };
 
 constexpr uint32_t kCutSeed = 0x9747b28cu; // second murmur seed: the pair is the 64-bit key identity of the memtable cut
 
+template <bool kClassIn>
 __global__ void __launch_bounds__(kRouteThreads) k_route_hash(RouteParams p) {
     pdl_trigger();
     pdl_wait();
@@ -51,7 +56,19 @@ __global__ void __launch_bounds__(kRouteThreads) k_route_hash(RouteParams p) {
     for (uint32_t s = tid; s < p.n_shards; s += kRouteThreads) { s_cnt[s] = 0; s_bytes[s] = 0; }
     __syncthreads();
     const uint32_t i = blockIdx.x * (uint32_t)kRouteThreads + tid;
-    if (i < p.n) {
+    if (kClassIn) {
+        if (i < p.n) {
+            uint32_t c = p.shard_of[i];
+            if (c != 0xFFFFFFFFu && (unsigned long long)i >= (*p.stop >> 2)) { // behind the record that ends the scan
+                c = 0xFFFFFFFFu;
+                p.shard_of[i] = c;
+            }
+            if (c != 0xFFFFFFFFu) {
+                atomicAdd(&s_cnt[c], 1u);
+                atomicAdd(&s_bytes[c], (unsigned long long)__ldg(&p.index[i]).w);
+            }
+        }
+    } else if (i < p.n) {
         const uint4 rec = __ldg(&p.index[i]);
         const uint64_t off = (uint64_t)rec.x | ((uint64_t)rec.y << 32);
         uint32_t owner = 0xFFFFFFFFu;

@@ -48,6 +48,9 @@ def _lib():
                                               C.POINTER(C.c_uint64), C.POINTER(C.c_int32), C.c_char_p]
         L.dbeel_tree_get_many.restype = C.c_int
         L.dbeel_tree_get_many.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p]
+        L.dbeel_tree_scan_ranges.restype = C.c_int
+        L.dbeel_tree_scan_ranges.argtypes = [C.c_void_p, C.POINTER(capi.Run), C.c_uint32, C.POINTER(capi.HashRange), C.c_uint32,
+                                             C.c_uint32, C.POINTER(capi.Out), C.POINTER(capi.FlushTable), C.POINTER(capi.ScanStop)]
         L.dbeel_tree_recover_wal.restype = C.c_int
         L.dbeel_tree_recover_wal.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.dbeel_tree_last_error.restype = C.c_char_p
@@ -67,7 +70,7 @@ def _lib():
 
 
 TREE_EXPORTS = ["dbeel_tree_open", "dbeel_tree_close", "dbeel_tree_sstables", "dbeel_tree_write_sstable_index",
-                "dbeel_tree_compact", "dbeel_tree_compact_many", "dbeel_tree_flush", "dbeel_tree_recover_wal", "dbeel_tree_get_many", "dbeel_tree_last_error", "dbeel_memtable_cut",
+                "dbeel_tree_compact", "dbeel_tree_compact_many", "dbeel_tree_flush", "dbeel_tree_recover_wal", "dbeel_tree_get_many", "dbeel_tree_scan_ranges", "dbeel_tree_last_error", "dbeel_memtable_cut",
                 "dbeel_plan_compactions", "dbeel_out_pages", "dbeel_tree_set_page_sink"]
 
 
@@ -184,6 +187,30 @@ class LSMTree:
             o, ks, fs = int.from_bytes(rec[:8], "little"), int.from_bytes(rec[8:12], "little"), int.from_bytes(rec[12:], "little")
             out.append(bytes(d[o + ks + 8:o + fs - 16]))  # EntryValue.data (entry = key | dlen | data | ts)
         return out
+
+    def scan_ranges(self, ranges: Sequence[Tuple[int, int]], mode: int = capi.SCAN_REFERENCE, memtables=()):
+        """The scan of migrate_actions (migration.rs:62-131) over this tree: every entry whose murmur3_32(key) lies in
+        one of `ranges`, assigned to the first range that holds.  memtables: (data, index) sorted runs of the flushing
+        and then the active memtable.  Returns (data, index, per_range, stop) like capi.Engine.scan_ranges, stop's table
+        counting the SSTables in sstable_indices_and_sizes() order and then `memtables`."""
+        from . import sstable
+        keep = [(capi._u8(d), capi._u8(i)) for d, i in memtables]
+        mts = (capi.Run * max(1, len(keep)))()
+        for j, (d, i) in enumerate(keep):
+            mts[j] = capi.Run(d.ctypes.data, d.size, i.ctypes.data, i.size)
+        dc = sum(d.size for d, _ in keep)
+        ic = 16 * sum(i.size // 16 for _, i in keep)
+        for idx, size in self.sstable_indices_and_sizes():
+            d, i = sstable.read_run_files(self.dir, idx)
+            dc += len(d)
+            ic += 16 * (len(i) // 16)
+        od, oi = np.empty(max(1, dc), np.uint8), np.empty(max(1, ic), np.uint8)
+        out = capi.Out(od.ctypes.data, dc, 0, oi.ctypes.data, ic, 0, None, 0, 0, 0)
+        rng, per_range, stop = capi.Engine._scan_args(ranges)
+        self._check(_lib().dbeel_tree_scan_ranges(self._h, mts, len(keep), rng, len(ranges), mode, C.byref(out), per_range,
+                                                  C.byref(stop)), "LSMTree.scan_ranges")
+        rows, st = capi.Engine._scan_result(per_range, len(ranges), stop)
+        return od[:out.data_len], oi[:out.index_len], rows, st
 
     def recover_wal(self, tree_capacity: int = capi.DEFAULT_TREE_CAPACITY) -> Tuple[int, int]:
         """open_or_create_ex's WAL step (lsm_tree.rs:466-513): with two `.memtable` files the older one is replayed and

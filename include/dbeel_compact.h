@@ -341,6 +341,62 @@ int dbeel_get_many_device(dbeel_engine *e, const dbeel_table *tables, uint32_t n
 int dbeel_wal_flush(dbeel_engine *e, const void *wal, uint64_t wal_len, uint32_t capacity, dbeel_out *out);
 int dbeel_wal_flush_device(dbeel_engine *e, const void *wal, uint64_t wal_len, uint32_t capacity, dbeel_out *out);
 
+/* ---- hash-range scans: the iterator behind shard migration -----------------------------------------------------
+ * Replaces the scan of migrate_actions (src/tasks/migration.rs:62-131): LSMTree::iter_filter (lsm_tree.rs:133-282) over
+ * the whole tree, keeping every entry whose murmur3_32(key bytes, seed 0) lies in one of `ranges` and assigning it to the
+ * FIRST range that holds (between_cmp, migration.rs:54-60; `position`, :98-104).  Range planning, the sends and the
+ * deletes stay with the caller.
+ *
+ * tables[] lists the tables in iteration order: for a live tree its SSTables oldest first (ascending file index), then
+ * the flushing memtable and then the active memtable, each as a sorted run-layout buffer (what dbeel_flush would write
+ * for it).  Every table's records are visited 0 .. index_len/16 - 1 (a ragged tail is ignored); nothing is deduplicated,
+ * so old versions and tombstones are yielded wherever they lie.  Every record is read the way AsyncIter::read_one reads
+ * it: the full_size bytes at its `offset` (key_size is ignored) must deserialize as exactly one Entry, timestamp in range.
+ *
+ * The scan ends at the first record it cannot yield, like the reference's `while let Ok(Some(entry))` (:96): nothing
+ * after it -- later tables and memtables included -- is selected.  *stop says where:
+ *   DBEEL_SCAN_DECODE  a bincode or timestamp failure (the reference's loop ends silently there);
+ *   DBEEL_SCAN_READ    full_size == 0, bytes past the end of .data, or a table with no record (its first index read hits
+ *                      EOF; leave EMPTY MEMTABLES out of tables[] -- the reference iterates them without reading).  The
+ *                      reference panics on these; whether a read past EOF panics there depends on whether the zero-padded
+ *                      last page is in its page cache, and this engine always stops.
+ *
+ *   DBEEL_SCAN_REFERENCE  between_cmp read literally: a wrapped range (end < start) holds for every hash, start == end
+ *                         for none.  Node removal and step 1 of node addition pass (previous shard, this shard), which
+ *                         wraps for the lowest shard on the ring.
+ *   DBEEL_SCAN_EXACT      a wrapped range is [start, 2^32) u [0, end).
+ *
+ * Output: range r's entries, in iteration order, back to back in out->data / out->index at per_range[r] (n_ranges rows,
+ * host memory).  Every range's .index carries offsets relative to its own .data (key_size = 8 + klen, full_size), so
+ * every range's output is both a valid SSTable-layout run and a valid arrival batch for dbeel_flush on the receiving
+ * shard.  No bloom (bloom_cap is ignored).  data_cap >= sum(data_len) and index_cap >= 16 * records always suffice;
+ * smaller caps that the selection does not fit give DBEEL_ERR_CAPACITY (nothing is written) with *stop filled in.
+ * n_ranges > DBEEL_MAX_SCAN_RANGES: DBEEL_ERR_INVALID_ARG.  Zero tables or zero ranges: empty outputs.
+ * dbeel_last_stats: ms_extract = classify, ms_resolve = split by range + offsets, ms_gather = payload copy.
+ *
+ * dbeel_scan_ranges takes host buffers and uploads every table whole (the tree must fit in device memory; nothing is
+ * streamed); dbeel_scan_ranges_device takes tables and out in device memory (.index and outputs 16-byte aligned), ranges /
+ * per_range / stop in host memory. */
+#define DBEEL_SCAN_REFERENCE 0u
+#define DBEEL_SCAN_EXACT 1u
+#define DBEEL_MAX_SCAN_RANGES 256u
+#define DBEEL_SCAN_END 0u    /* ran to the end of the last table          */
+#define DBEEL_SCAN_DECODE 1u /* stopped: the reference's loop ends here   */
+#define DBEEL_SCAN_READ 2u   /* stopped: the reference panics here        */
+typedef struct dbeel_hash_range {
+    uint32_t start, end;
+} dbeel_hash_range;
+typedef struct dbeel_scan_stop {
+    int32_t table;   /* position in tables[] of the record that stopped the scan, -1: DBEEL_SCAN_END */
+    uint32_t reason; /* DBEEL_SCAN_*                                                              */
+    uint64_t record; /* its record number inside that table                                       */
+} dbeel_scan_stop;
+int dbeel_scan_ranges(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges,
+                      uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range, dbeel_scan_stop *stop);
+int dbeel_scan_ranges_device(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges,
+                             uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range,
+                             dbeel_scan_stop *stop);
+
 /* Bloom::new_for_fp_rate arithmetic (bloomfilter 1.0.12). */
 uint64_t dbeel_bloom_bitmap_bytes(uint64_t items, double fp);
 uint32_t dbeel_bloom_k_num(uint64_t bitmap_bits, uint64_t items);

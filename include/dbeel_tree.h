@@ -17,6 +17,8 @@
  *                             next even index through dbeel_flush(), no bloom
  *   dbeel_tree_sstables    <- LSMTree::sstable_indices_and_sizes (lsm_tree.rs:592-598)
  *   dbeel_tree_get_many    <- the SSTable loop of LSMTree::get_entry (lsm_tree.rs:686-719) through dbeel_get_many()
+ *   dbeel_tree_scan_ranges <- migrate_actions' scan over iter_filter (src/tasks/migration.rs:62-131) through
+ *                             dbeel_scan_ranges()
  *   dbeel_memtable_cut     <- RedBlackTree::set + active_memtable_full (rbtree_arena lib.rs:497-534,
  *                             lsm_tree.rs:600-603,757-765): how many arrivals fill one memtable
  *   dbeel_plan_compactions <- compact_tree's size-tiered picker (src/tasks/compaction.rs:35-102),
@@ -75,6 +77,14 @@ int dbeel_tree_flush(dbeel_tree *t, const dbeel_run *batch, uint64_t *written_in
  * rows as in dbeel_get_many.  The memtable look-ups in front of it (:677-684) are the caller's. */
 int dbeel_tree_get_many(dbeel_tree *t, const void *keys, const uint64_t *key_offsets, uint64_t n_keys, uint32_t mode,
                         dbeel_lookup_result *results);
+
+/* The scan of migrate_actions (src/tasks/migration.rs:62-131) over this tree through dbeel_scan_ranges(): the tree's
+ * SSTables in dbeel_tree_sstables() order, then the caller's memtables (the flushing one, then the active one, each as a
+ * sorted run: this mirror keeps no memtable; empty ones are skipped).  stop->table is a position in that combined order
+ * (SSTables first, then memtables[]).  Ranges / modes / outputs as in dbeel_scan_ranges. */
+int dbeel_tree_scan_ranges(dbeel_tree *t, const dbeel_run *memtables, uint32_t n_memtables, const dbeel_hash_range *ranges,
+                           uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range,
+                           dbeel_scan_stop *stop);
 
 /* WAL recovery step of open_or_create_ex.  0 logs: *wal_file_index = 0; 1 log: its index; 2 logs: the older one is
  * replayed (memtable of `tree_capacity` entries, DBEEL_ERR_TREE_FULL like the reference's ReachedCapacity), flushed
