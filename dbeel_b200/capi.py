@@ -44,7 +44,7 @@ EXPORTS = ["dbeel_abi_version", "dbeel_engine_create", "dbeel_engine_destroy", "
            "dbeel_host_free", "dbeel_last_stats", "dbeel_last_error", "dbeel_strerror",
            "dbeel_murmur3_32", "dbeel_ring_owner", "dbeel_shard_ring", "dbeel_route_device", "dbeel_flush_many_sparse_device",
            "dbeel_gpu_numa_node", "dbeel_bind_to_gpu", "dbeel_memtable_cuts_device", "dbeel_engine_stream",
-           "dbeel_scan_ranges", "dbeel_scan_ranges_device"]
+           "dbeel_scan_ranges", "dbeel_scan_ranges_device", "dbeel_scan_ranges_stream"]
 
 
 class Run(C.Structure):
@@ -57,6 +57,14 @@ STREAM_WRITE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint64, C.c_v
 
 class StreamIO(C.Structure):
     _fields_ = [("read", STREAM_READ_FN), ("write", STREAM_WRITE_FN), ("ctx", C.c_void_p)]
+
+
+SCAN_READ_FN = STREAM_READ_FN  # (ctx, table, kind, offset, len, dst)
+SCAN_WRITE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p, C.c_uint64)  # (ctx, range, kind, ...)
+
+
+class ScanIO(C.Structure):
+    _fields_ = [("read", SCAN_READ_FN), ("write", SCAN_WRITE_FN), ("ctx", C.c_void_p)]
 
 
 class Out(C.Structure):
@@ -234,6 +242,9 @@ def lib():
             f.restype = C.c_int
             f.argtypes = [C.c_void_p, C.POINTER(Run), C.c_uint32, C.POINTER(HashRange), C.c_uint32, C.c_uint32, C.POINTER(Out),
                           C.POINTER(FlushTable), C.POINTER(ScanStop)]
+        L.dbeel_scan_ranges_stream.restype = C.c_int
+        L.dbeel_scan_ranges_stream.argtypes = [C.c_void_p, C.POINTER(Run), C.c_uint32, C.POINTER(HashRange), C.c_uint32, C.c_uint32,
+                                               C.POINTER(ScanIO), C.c_uint64, C.POINTER(FlushTable), C.POINTER(ScanStop)]
         _lib = L
     return _lib
 
@@ -617,6 +628,62 @@ class Engine:
                                             C.byref(stop)), "dbeel_scan_ranges")
         rows, st = self._scan_result(per_range, len(ranges), stop)
         return od[:out.data_len], oi[:out.index_len], rows, st
+
+    def scan_ranges_stream(self, tables: Sequence[Tuple[object, object]], ranges: Sequence[Tuple[int, int]],
+                           mode: int = SCAN_REFERENCE, partition_bytes: int = 0, read_hook=None, write_hook=None):
+        """dbeel_scan_ranges_stream with in-memory "files": the engine pulls the tables through a read callback and pushes
+        every range's stream through a write callback (both called from several engine threads).  Returns (data, index,
+        per_range, stop) like scan_ranges(): the range streams concatenated in range order, per_range rebased to that
+        concatenation.  read_hook(table, kind, offset, len) / write_hook(range, kind, offset, len), when given, run before
+        every call; a nonzero return is what the callback returns (tests)."""
+        import threading
+        keep = [(_u8(d), _u8(i)) for d, i in tables]
+        arr = (Run * max(1, len(keep)))()
+        for j, (d, i) in enumerate(keep):
+            arr[j] = Run(None, d.size, None, i.size)
+        streams = {}  # (range, kind) -> bytearray
+        mu = threading.Lock()
+
+        def rd(_ctx, table, kind, off, n, dst):
+            if read_hook is not None:
+                rc = read_hook(table, kind, off, n)
+                if rc:
+                    return rc
+            src = keep[table][0] if kind == 1 else keep[table][1]
+            if off + n > src.size:
+                return 4243
+            C.memmove(dst, src.ctypes.data + off, n)
+            return 0
+
+        def wr(_ctx, rng_, kind, off, src, n):
+            if write_hook is not None:
+                rc = write_hook(rng_, kind, off, n)
+                if rc:
+                    return rc
+            if kind not in (1, 2) or rng_ >= len(ranges):
+                return 4244
+            b = C.string_at(src, n)
+            with mu:
+                buf = streams.setdefault((rng_, kind), bytearray())
+                if len(buf) < off + n:
+                    buf.extend(bytes(off + n - len(buf)))
+                buf[off:off + n] = b
+            return 0
+
+        io = ScanIO(SCAN_READ_FN(rd), SCAN_WRITE_FN(wr), None)
+        rng, per_range, stop = self._scan_args(ranges)
+        self._check(lib().dbeel_scan_ranges_stream(self._h, arr, len(keep), rng, len(ranges), mode, C.byref(io), partition_bytes,
+                                                   per_range, C.byref(stop)), "dbeel_scan_ranges_stream")
+        rows, st = self._scan_result(per_range, len(ranges), stop)
+        data, index = bytearray(), bytearray()
+        for r, row in enumerate(rows):
+            d, i = bytes(streams.get((r, 1), b"")), bytes(streams.get((r, 2), b""))
+            if len(d) != row["data_len"] or len(i) != row["index_len"] or row["data_off"] or row["index_off"]:
+                raise AssertionError(f"range {r}: stream of {len(d)} / {len(i)} bytes against per_range {row}")
+            row["data_off"], row["index_off"] = len(data), len(index)
+            data += d
+            index += i
+        return np.frombuffer(bytes(data), np.uint8), np.frombuffer(bytes(index), np.uint8), rows, st
 
     def scan_ranges_device(self, tables: Sequence[Tuple[int, int, int, int]], ranges: Sequence[Tuple[int, int]],
                            out_ptrs: Tuple[int, int, int, int], mode: int = SCAN_REFERENCE):

@@ -28,6 +28,7 @@
 #include "route.cuh"
 #include "scan.cuh"
 #include "wal.cuh"
+#include "host/scan_plan.h"
 #include "host/stream_pump.h"
 
 using namespace dbeel;
@@ -2086,6 +2087,350 @@ int scan_entry(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, cons
     return DBEEL_OK;
 }
 
+// ------------------------------------------------------------------------------------ streamed hash-range scans
+// dbeel_scan_ranges_stream: the tables come through the read callback one partition at a time (host/scan_plan.h), every
+// range's output leaves through the write callback as its own stream.  Per partition c:
+//   reader threads   c's .data spans -> pinned ring slot c mod R (the .index files are read whole first: the plan needs them)
+//   engine thread    H2D of c's spans and index slices -> device buffer c & 1; the scan kernels over c's records; the
+//                    exact-size D2H of c's range-major output -> pinned output slot c mod R, once c's header has arrived
+//   writer threads   every range's piece of c -> the write callback, at the range's running stream offsets
+// The engine enqueues c + 1's kernels before it waits for c's header, so the copies and the kernels keep overlapping; the
+// stop word and the running per-range totals live on the device (k_scan_part_enter / _leave), so the kernels of c + 1
+// never depend on the host having seen c.
+int scan_stream_entry(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges, uint32_t n_ranges,
+                      uint32_t mode, const dbeel_scan_io *io, uint64_t partition_bytes, dbeel_flush_table *per_range, dbeel_scan_stop *stop) {
+    if (!e) return DBEEL_ERR_INVALID_ARG;
+    if (!stop || !io || !io->read || !io->write || (n_tables && !tables) || (n_ranges && (!ranges || !per_range)))
+        return fail(e, DBEEL_ERR_INVALID_ARG, "null argument");
+    if (mode > DBEEL_SCAN_EXACT) return fail(e, DBEEL_ERR_INVALID_ARG, "unknown scan mode");
+    if (n_ranges > DBEEL_MAX_SCAN_RANGES) return fail(e, DBEEL_ERR_INVALID_ARG, "more than DBEEL_MAX_SCAN_RANGES ranges");
+    if (e->busy) return fail(e, DBEEL_ERR_BUSY, "engine busy");
+    BusyGuard g(e);
+    e->err.clear();
+    e->stats = dbeel_stats{};
+    dbeel_stats &st = e->stats;
+    for (uint32_t r = 0; r < n_ranges; r++) per_range[r] = dbeel_flush_table{0, 0, 0, 0, 0};
+    *stop = dbeel_scan_stop{-1, DBEEL_SCAN_END, 0};
+    cudaError_t ce = cudaSetDevice(e->device);
+    if (ce != cudaSuccess) return fail(e, DBEEL_ERR_CUDA, "cudaSetDevice", ce);
+    const uint64_t budget = partition_bytes ? partition_bytes : e->partition_bytes;
+
+    // ---- 1. the .index files of the tables in front of the first one without a record, whole, into page-locked memory
+    uint32_t nt = 0;
+    uint64_t need = 0;
+    std::vector<uint64_t> ioff, tbase; // pinned offset of table t's .index; ordinal of its record 0
+    while (nt < n_tables && tables[nt].index_len >= DBEEL_INDEX_ENTRY_SIZE) {
+        ioff.push_back(need);
+        tbase.push_back(st.entries_in);
+        need += align_up(tables[nt].index_len / 16 * 16 + 16, kAlign);
+        st.entries_in += tables[nt].index_len / DBEEL_INDEX_ENTRY_SIZE;
+        st.input_bytes += tables[nt].data_len + tables[nt].index_len;
+        nt++;
+    }
+    int rc = ensure_host(e, &e->pin_index, &e->pin_index_cap, std::max<uint64_t>(need, 256));
+    if (rc) return rc;
+    {
+        std::vector<StreamPump::ReadTask> rt;
+        for (uint32_t t = 0; t < nt; t++)
+            for (uint64_t d = 0, n = tables[t].index_len / 16 * 16; d < n; d += StreamPump::kPiece)
+                rt.push_back(StreamPump::ReadTask{0, t, DBEEL_STREAM_INDEX, d, std::min<uint64_t>(StreamPump::kPiece, n - d), e->pin_index + ioff[t] + d});
+        rc = parallel_pieces(rt.size(), [&](size_t k) { return io->read(io->ctx, rt[k].run, rt[k].kind, rt[k].off, rt[k].len, rt[k].dst); });
+        if (rc) return fail(e, rc, "scan read callback failed (.index)");
+    }
+
+    // ---- 2. the plan (it schedules nothing at or after the first READ stop)
+    std::vector<ScanPlanTable> pt(nt);
+    for (uint32_t t = 0; t < nt; t++) pt[t] = ScanPlanTable{tables[t].data_len, e->pin_index + ioff[t], tables[t].index_len / DBEEL_INDEX_ENTRY_SIZE};
+    const ScanPlan plan = scan_plan(pt.data(), nt, budget);
+    // table t stops the scan at record r when the scan gets there: as nt < n_tables (an empty table) or the plan found
+    if (plan.stopped) *stop = dbeel_scan_stop{(int32_t)plan.stop_table, DBEEL_SCAN_READ, plan.stop_record};
+    else if (nt < n_tables) *stop = dbeel_scan_stop{(int32_t)nt, DBEEL_SCAN_READ, 0};
+    st.entries_valid = plan.scheduled;
+    const uint32_t np = (uint32_t)plan.parts.size();
+    if (np == 0) return DBEEL_OK;
+
+    // ---- 3. slot layouts: every piece's span (+32 bytes of slack for the narrow loads, aligned), then its index slice
+    auto span_room = [](const ScanPiece &k) { return align_up(k.span_hi - k.span_lo + 32, kAlign); };
+    auto slice_room = [](const ScanPiece &k) { return align_up(16 * (k.rec_hi - k.rec_lo) + 16, kAlign); };
+    uint64_t max_in = 0, max_out = 0, max_n = 0, max_tiles = 0;
+    for (const ScanPart &q : plan.parts) {
+        uint64_t in = 0;
+        for (uint32_t k = q.first_piece; k < q.first_piece + q.n_pieces; k++) in += span_room(plan.pieces[k]) + slice_room(plan.pieces[k]);
+        max_in = std::max(max_in, in);
+        max_out = std::max(max_out, align_up(q.data_bytes + 16, kAlign) + align_up(16 * q.records + 16, kAlign));
+        max_n = std::max(max_n, q.records);
+        max_tiles = std::max<uint64_t>(max_tiles, (q.data_bytes + kGatherTileBytes - 1) / kGatherTileBytes);
+    }
+    const uint32_t n_cls = n_ranges ? n_ranges : 1; // no ranges: one class that selects nothing, so the stop is still found
+    const uint32_t NM = (uint32_t)max_n;
+    const uint64_t blocks_max = (NM + kRouteThreads - 1) / kRouteThreads;
+    const uint64_t tiles_max = (NM + kResolveThreads - 1) / kResolveThreads, chunks_max = (tiles_max + 1023) / 1024;
+    uint64_t off = 0;
+    auto carve = [&](uint64_t b) { uint64_t o2 = off; off = align_up(off + b, kAlign); return o2; };
+    const uint64_t o_tab = carve(sizeof(ScanTable) * plan.pieces.size()), o_rng = carve(8ull * n_cls), o_ctl = carve(sizeof(Ctl));
+    const uint64_t o_mt = carve(16ull * (n_cls + 1)), o_lstop = carve(8), o_gstop = carve(8), o_run = carve(16ull * n_cls);
+    const uint64_t o_seg = carve(sizeof(Seg) * n_cls), o_tot = carve(8ull * (3 * n_cls + 1)), o_rtot = carve(8ull * (3 * n_cls + 1));
+    const uint64_t o_hist = carve(4ull * blocks_max * n_cls);
+    const uint64_t o_cls = carve(4ull * NM), o_rec = carve(16ull * NM), o_res = carve(16ull * NM), o_src = carve(8ull * NM);
+    const uint64_t o_tb = carve(8 * tiles_max), o_tc = carve(4 * tiles_max), o_cb = carve(8 * chunks_max), o_cc = carve(4 * chunks_max);
+    const uint64_t o_tf = carve(4ull * (max_tiles + 2));
+    const uint64_t hdr_stride = align_up(8 + sizeof(ScanPieceRow) * n_cls, 64);
+    const uint32_t R = (uint32_t)std::max(2, e->stream_ring);
+    rc = ensure_device(e, &e->ws, &e->ws_cap, off);
+    if (!rc) rc = ensure_device(e, &e->stage_in, &e->stage_in_cap, max_in);
+    if (!rc) rc = ensure_device(e, &e->stage_in2, &e->stage_in2_cap, max_in);
+    if (!rc) rc = ensure_device(e, &e->stage_out, &e->stage_out_cap, max_out);
+    if (!rc) rc = ensure_device(e, &e->stage_out2, &e->stage_out2_cap, max_out);
+    if (!rc) rc = ensure_pinned(e, 2 * hdr_stride);
+    if (!rc) rc = ensure_host(e, &e->ring_in, &e->ring_in_cap, (uint64_t)R * max_in);
+    if (!rc) rc = ensure_host(e, &e->ring_out, &e->ring_out_cap, (uint64_t)R * max_out);
+    if (rc) return rc;
+    if (!e->s_h2d) {
+        CU(cudaStreamCreateWithFlags(&e->s_h2d, cudaStreamNonBlocking));
+        CU(cudaStreamCreateWithFlags(&e->s_d2h, cudaStreamNonBlocking));
+        for (int i = 0; i < 2; i++) {
+            CU(cudaEventCreateWithFlags(&e->ev_h2d[i], cudaEventDisableTiming));
+            CU(cudaEventCreateWithFlags(&e->ev_comp[i], cudaEventDisableTiming));
+            CU(cudaEventCreateWithFlags(&e->ev_d2h[i], cudaEventDisableTiming));
+        }
+    }
+    uint8_t *ws = e->ws, *sin[2] = {e->stage_in, e->stage_in2}, *sout[2] = {e->stage_out, e->stage_out2};
+    cudaStream_t s = e->stream;
+
+    // every partition's ScanTables (device input buffer c & 1 is known in advance), the ranges, the cross-partition state
+    std::vector<ScanTable> ht(plan.pieces.size());
+    std::vector<std::vector<uint64_t>> span_at(np); // slot offset of every piece's span
+    for (uint32_t c = 0; c < np; c++) {
+        const ScanPart &q = plan.parts[c];
+        uint64_t pos = 0;
+        for (uint32_t k = q.first_piece; k < q.first_piece + q.n_pieces; k++) {
+            const ScanPiece &pc = plan.pieces[k];
+            span_at[c].push_back(pos);
+            const uint8_t *span = sin[c & 1] + pos;
+            pos += span_room(pc);
+            ht[k] = ScanTable{span - pc.span_lo, tables[pc.table].data_len, reinterpret_cast<const uint4 *>(sin[c & 1] + pos),
+                              (uint32_t)(tbase[pc.table] + pc.rec_lo - q.first_ordinal), (uint32_t)(pc.rec_hi - pc.rec_lo)};
+            pos += slice_room(pc);
+        }
+    }
+    std::vector<uint2> hr(n_cls, make_uint2(0, 0)); // no ranges: start == end holds for no hash in either mode
+    for (uint32_t r = 0; r < n_ranges; r++) hr[r] = make_uint2(ranges[r].start, ranges[r].end);
+    CU(cudaMemcpyAsync(ws + o_tab, ht.data(), sizeof(ScanTable) * ht.size(), cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(ws + o_rng, hr.data(), 8ull * n_cls, cudaMemcpyHostToDevice, s));
+    CU(cudaMemsetAsync(ws + o_gstop, 0xFF, 8, s));
+    CU(cudaMemsetAsync(ws + o_run, 0, 16ull * n_cls, s));
+    CU(cudaStreamSynchronize(s)); // ht / hr are pageable
+
+    // the pump: R-slot pinned rings, one event per partition for the writer threads.  Declared in this order so that the
+    // pump's threads are joined before the events they wait on are destroyed.
+    struct EventList {
+        std::vector<cudaEvent_t> ev;
+        ~EventList() { for (auto &x : ev) if (x) cudaEventDestroy(x); }
+    } ev_out;
+    ev_out.ev.assign(np, nullptr);
+    for (uint32_t c = 0; c < np; c++) CU(cudaEventCreateWithFlags(&ev_out.ev[c], cudaEventDisableTiming | cudaEventBlockingSync));
+    // per device buffer: begin / end of the H2D copies, the kernels and the D2H copies of the partition that last used it
+    EventList tev;
+    tev.ev.assign(12, nullptr);
+    for (auto &x : tev.ev) CU(cudaEventCreate(&x));
+    enum { T_H2D = 0, T_KER = 4, T_D2H = 8 };
+    auto stage_ms = [&](int stage, uint32_t slot) {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, tev.ev[stage + 2 * slot], tev.ev[stage + 2 * slot + 1]);
+        return ms;
+    };
+    const dbeel_stream_io rio{io->read, nullptr, io->ctx};
+    const int dev = e->device;
+    EventList *evl = &ev_out;
+    std::unique_ptr<StreamPump> pump(new StreamPump(&rio, np, R, stream_threads(), [evl](uint32_t c) { cudaEventSynchronize(evl->ev[c]); },
+                                                    [dev]() { cudaSetDevice(dev); }));
+    pump->set_stream_write(io->write);
+    for (uint32_t c = 0; c < np; c++) {
+        const ScanPart &q = plan.parts[c];
+        uint8_t *slot = e->ring_in + (uint64_t)(c % R) * max_in;
+        for (uint32_t j = 0; j < q.n_pieces; j++) {
+            const ScanPiece &pc = plan.pieces[q.first_piece + j];
+            pump->add_read(c, pc.table, DBEEL_STREAM_DATA, pc.span_lo, pc.span_hi - pc.span_lo, slot + span_at[c][j]);
+        }
+    }
+    pump->start();
+
+    auto enqueue_h2d = [&](uint32_t c) -> int {
+        const int prc = pump->wait_reads(c);
+        if (prc) return fail(e, prc, "scan read callback failed (.data)");
+        const ScanPart &q = plan.parts[c];
+        const uint8_t *slot = e->ring_in + (uint64_t)(c % R) * max_in;
+        CU(cudaEventRecord(tev.ev[T_H2D + 2 * (c & 1)], e->s_h2d));
+        for (uint32_t j = 0; j < q.n_pieces; j++) {
+            const ScanPiece &pc = plan.pieces[q.first_piece + j];
+            const uint64_t sl = pc.span_hi - pc.span_lo, il = 16 * (pc.rec_hi - pc.rec_lo), at = span_at[c][j];
+            CU(cudaMemcpyAsync(sin[c & 1] + at, slot + at, sl, cudaMemcpyHostToDevice, e->s_h2d));
+            CU(cudaMemcpyAsync(sin[c & 1] + at + span_room(pc), e->pin_index + ioff[pc.table] + 16 * pc.rec_lo, il, cudaMemcpyHostToDevice, e->s_h2d));
+        }
+        CU(cudaEventRecord(tev.ev[T_H2D + 2 * (c & 1) + 1], e->s_h2d));
+        CU(cudaEventRecord(e->ev_h2d[c & 1], e->s_h2d));
+        return DBEEL_OK;
+    };
+    uint32_t launches = 0;
+    auto enqueue_kernels = [&](uint32_t c) -> int {
+        const ScanPart &q = plan.parts[c];
+        const uint32_t N = (uint32_t)q.records;
+        const uint32_t n_blocks = (N + kRouteThreads - 1) / kRouteThreads;
+        const uint64_t res_tiles = (N + kResolveThreads - 1) / kResolveThreads, res_chunks = (res_tiles + 1023) / 1024;
+        const uint64_t gather_tiles = (q.data_bytes + kGatherTileBytes - 1) / kGatherTileBytes;
+        uint8_t *od = sout[c & 1], *oi = sout[c & 1] + align_up(q.data_bytes + 16, kAlign);
+        ScanParams sp;
+        sp.tables = reinterpret_cast<const ScanTable *>(ws + o_tab) + q.first_piece;
+        sp.n_tables = q.n_pieces;
+        sp.n = N;
+        sp.ranges = reinterpret_cast<const uint2 *>(ws + o_rng);
+        sp.n_ranges = n_cls;
+        sp.mode = mode;
+        sp.cls = reinterpret_cast<uint32_t *>(ws + o_cls);
+        sp.rec = reinterpret_cast<uint4 *>(ws + o_rec);
+        sp.stop = reinterpret_cast<unsigned long long *>(ws + o_lstop);
+        sp.totals = reinterpret_cast<unsigned long long *>(ws + o_tot);
+        sp.ctl = reinterpret_cast<Ctl *>(ws + o_ctl);
+        sp.seg = reinterpret_cast<Seg *>(ws + o_seg);
+        sp.data_cap = q.data_bytes;
+        sp.index_cap = 16ull * N;
+        RouteParams rp;
+        memset(&rp, 0, sizeof rp);
+        rp.index = sp.rec;
+        rp.n = N;
+        rp.n_shards = n_cls;
+        rp.n_blocks = n_blocks;
+        rp.shard_of = sp.cls;
+        rp.hist = reinterpret_cast<uint32_t *>(ws + o_hist);
+        rp.totals = sp.totals;
+        rp.out_index = reinterpret_cast<uint4 *>(ws + o_res);
+        rp.stop = sp.stop;
+        Params p;
+        memset(&p, 0, sizeof p);
+        p.n_total = N;
+        p.ctl = sp.ctl;
+        p.seg[0] = sp.seg;
+        p.n_groups = n_cls;
+        p.mem_table = reinterpret_cast<unsigned long long *>(ws + o_mt);
+        p.tile_bytes = reinterpret_cast<unsigned long long *>(ws + o_tb);
+        p.tile_count = reinterpret_cast<uint32_t *>(ws + o_tc);
+        p.chunk_bytes = reinterpret_cast<unsigned long long *>(ws + o_cb);
+        p.chunk_count = reinterpret_cast<uint32_t *>(ws + o_cc);
+        p.src_ptr = reinterpret_cast<unsigned long long *>(ws + o_src);
+        p.tile_first = reinterpret_cast<uint32_t *>(ws + o_tf);
+        p.tile_first_n = (uint32_t)(gather_tiles + 2);
+        p.out_data = od;
+        p.out_index = reinterpret_cast<uint4 *>(oi);
+        const uint4 *res = rp.out_index;
+        CU(cudaStreamWaitEvent(s, e->ev_h2d[c & 1], 0));
+        if (c >= 2) CU(cudaStreamWaitEvent(s, e->ev_d2h[c & 1], 0)); // output buffer c & 1 drained by partition c - 2's D2H
+        CU(cudaEventRecord(tev.ev[T_KER + 2 * (c & 1)], s));
+        k_scan_part_enter<<<1, 1, 0, s>>>(sp.stop, reinterpret_cast<const unsigned long long *>(ws + o_gstop));
+        CU(cudaMemsetAsync(sp.ctl, 0, sizeof(Ctl), s));
+        CU(cudaMemsetAsync(sp.totals, 0, 8ull * (3 * n_cls + 1), s));
+        k_scan_classify<<<(N + 255) / 256, 256, 0, s>>>(sp);
+        k_route_hash<true><<<n_blocks, kRouteThreads, 0, s>>>(rp);
+        k_route_scan<<<n_cls, 1024, 0, s>>>(rp);
+        k_route_starts<<<1, 256, 0, s>>>(rp, reinterpret_cast<unsigned long long *>(ws + o_rtot));
+        k_route_scatter<<<n_blocks, kRouteThreads, 0, s>>>(rp);
+        k_scan_plan<<<1, 256, 0, s>>>(sp);
+        k_scan_res_tiles<<<(uint32_t)res_tiles, kResolveThreads, 0, s>>>(p, res);
+        k_scan_tiles<<<(uint32_t)res_chunks, 1024, 0, s>>>(p);
+        k_scan_chunks<<<1, 1024, 0, s>>>(p);
+        k_emit<<<(uint32_t)res_tiles, kResolveThreads, 0, s>>>(p, res);
+        k_flush_table<<<(n_cls + 1 + 127) / 128, 128, 0, s>>>(p, res);
+        launches += 13;
+        if (gather_tiles) {
+            if (((uintptr_t)od & 31) == 0) k_gather32<false, false, false, true><<<(uint32_t)gather_tiles, kGatherThreads, 0, s>>>(p);
+            else k_gather<<<(uint32_t)gather_tiles, kGatherThreads, 0, s>>>(p);
+            launches++;
+        }
+        k_scan_rebase_stream<<<(N + 255) / 256, 256, 0, s>>>(p, reinterpret_cast<const unsigned long long *>(ws + o_run)); // after the gather
+        k_scan_part_leave<<<1, 256, 0, s>>>(p.mem_table, n_ranges, sp.stop, reinterpret_cast<unsigned long long *>(ws + o_gstop), q.first_ordinal,
+                                            reinterpret_cast<unsigned long long *>(ws + o_run),
+                                            reinterpret_cast<unsigned long long *>(e->pin_dev + (c & 1) * hdr_stride));
+        launches += 2;
+        CU(cudaGetLastError());
+        CU(cudaEventRecord(tev.ev[T_KER + 2 * (c & 1) + 1], s));
+        CU(cudaEventRecord(e->ev_comp[c & 1], s));
+        return DBEEL_OK;
+    };
+
+    uint64_t out_data = 0, out_items = 0, gstop = ~0ull;
+    uint32_t done = 0; // partitions whose output has been published
+    std::vector<StreamPump::OutPiece> pieces;
+    rc = enqueue_h2d(0);
+    if (!rc && np > 1) rc = enqueue_h2d(1);
+    if (!rc) rc = enqueue_kernels(0);
+    for (uint32_t c = 0; c < np && !rc; c++) {
+        if (c + 1 < np && (rc = enqueue_kernels(c + 1))) break;
+        ce = cudaEventSynchronize(e->ev_comp[c & 1]);
+        if (ce != cudaSuccess) { rc = fail(e, DBEEL_ERR_CUDA, "scan partition kernels", ce); break; }
+        pump->release_input(c); // the kernels have read device buffer c & 1, which the H2D out of ring slot c mod R filled
+        st.ms_h2d += stage_ms(T_H2D, c & 1);
+        st.ms_total += stage_ms(T_KER, c & 1);
+        if (c >= 2) { // partition c - 2's D2H (the kernels of c waited for it)
+            CU(cudaEventSynchronize(tev.ev[T_D2H + 2 * (c & 1) + 1]));
+            st.ms_d2h += stage_ms(T_D2H, c & 1);
+        }
+        const unsigned long long *hdr = reinterpret_cast<const unsigned long long *>(e->pin + (c & 1) * hdr_stride);
+        const ScanPieceRow *rows = reinterpret_cast<const ScanPieceRow *>(hdr + 1);
+        gstop = hdr[0];
+        uint64_t dlen = 0, items = 0;
+        for (uint32_t r = 0; r < n_ranges; r++) { dlen += rows[r].data_len; items += rows[r].items; }
+        if ((rc = pump->wait_out_slot(c))) { fail(e, rc, "scan write callback failed"); break; }
+        uint8_t *oslot = e->ring_out + (uint64_t)(c % R) * max_out, *oindex = oslot + align_up(dlen + 16, kAlign);
+        const ScanPart &q = plan.parts[c];
+        CU(cudaStreamWaitEvent(e->s_d2h, e->ev_comp[c & 1], 0));
+        CU(cudaEventRecord(tev.ev[T_D2H + 2 * (c & 1)], e->s_d2h));
+        if (dlen) CU(cudaMemcpyAsync(oslot, sout[c & 1], dlen, cudaMemcpyDeviceToHost, e->s_d2h));
+        if (items) CU(cudaMemcpyAsync(oindex, sout[c & 1] + align_up(q.data_bytes + 16, kAlign), 16 * items, cudaMemcpyDeviceToHost, e->s_d2h));
+        CU(cudaEventRecord(tev.ev[T_D2H + 2 * (c & 1) + 1], e->s_d2h));
+        CU(cudaEventRecord(ev_out.ev[c], e->s_d2h));
+        CU(cudaEventRecord(e->ev_d2h[c & 1], e->s_d2h));
+        pieces.clear();
+        for (uint32_t r = 0; r < n_ranges; r++) {
+            const ScanPieceRow &w = rows[r];
+            if (w.data_len) pieces.push_back(StreamPump::OutPiece{oslot + w.data_at, w.data_len, r, DBEEL_STREAM_DATA, w.stream_data_off});
+            if (w.items) pieces.push_back(StreamPump::OutPiece{oindex + 16 * w.items_at, 16 * w.items, r, DBEEL_STREAM_INDEX, 16 * w.stream_items_off});
+            per_range[r].data_len += w.data_len;
+            per_range[r].items += w.items;
+        }
+        pump->publish_pieces(c, pieces);
+        done = c + 1;
+        out_data += dlen;
+        out_items += items;
+        if (gstop != ~0ull) { // the later partitions select nothing: read and write no more of them
+            pump->end_at(c + 1);
+            break;
+        }
+        if (c + 2 < np && (rc = enqueue_h2d(c + 2))) break;
+    }
+    cudaStreamSynchronize(s);
+    cudaStreamSynchronize(e->s_h2d);
+    cudaStreamSynchronize(e->s_d2h);
+    if (rc) {
+        pump->abort(rc); // its threads are joined when it goes out of scope
+        return rc;
+    }
+    const int frc = pump->finish(); // every published piece has gone through the write callback
+    if (frc) return fail(e, frc, "scan write callback failed");
+    for (uint32_t c = done >= 2 ? done - 2 : 0; c < done; c++) st.ms_d2h += stage_ms(T_D2H, c & 1); // the last two D2H
+    if (gstop != ~0ull) { // a DECODE stop (or a READ stop the device saw first) in front of the plan's
+        const uint64_t o = gstop >> 2;
+        uint32_t t = 0;
+        while (t + 1 < nt && tbase[t + 1] <= o) t++;
+        *stop = dbeel_scan_stop{(int32_t)t, (uint32_t)(gstop & 3), o - tbase[t]};
+        st.entries_valid = o;
+    }
+    for (uint32_t r = 0; r < n_ranges; r++) per_range[r].index_len = 16 * per_range[r].items;
+    st.entries_out = out_items;
+    st.output_bytes = out_data + 16 * out_items;
+    st.kernel_launches = launches;
+    st.partitions = done;
+    return DBEEL_OK;
+}
+
 } // namespace
 
 // ------------------------------------------------------------------------------------ C ABI
@@ -2440,6 +2785,13 @@ int dbeel_scan_ranges_device(dbeel_engine *e, const dbeel_run *tables, uint32_t 
                              uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range, dbeel_scan_stop *stop) {
     REFUSE_WHILE_ASYNC(e);
     return scan_entry(e, tables, n_tables, ranges, n_ranges, mode, out, per_range, stop, true);
+}
+
+int dbeel_scan_ranges_stream(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges,
+                             uint32_t n_ranges, uint32_t mode, const dbeel_scan_io *io, uint64_t partition_bytes,
+                             dbeel_flush_table *per_range, dbeel_scan_stop *stop) {
+    REFUSE_WHILE_ASYNC(e);
+    return scan_stream_entry(e, tables, n_tables, ranges, n_ranges, mode, io, partition_bytes, per_range, stop);
 }
 
 void *dbeel_host_alloc(uint64_t bytes) {

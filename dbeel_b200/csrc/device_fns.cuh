@@ -9,8 +9,10 @@
 
 #ifdef __CUDACC__
 #define DB_HD __device__ __forceinline__
+#define DB_HOST_HD __host__ __device__ __forceinline__ // also called by host code of the engine (host/scan_plan.h)
 #else
 #define DB_HD inline
+#define DB_HOST_HD inline
 #endif
 
 namespace dbeel {
@@ -360,7 +362,7 @@ DB_HD bool hash_in_range(uint32_t hash, uint32_t start, uint32_t end, uint32_t m
 // AsyncIter::read_one's read of one entry (lsm_tree.rs:250-262): read_at(offset, full_size) on the .data file.  The
 // reference asserts full_size != 0 (cached_file_reader.rs:82) and panics on bytes past the end of the file; both stop a
 // scan.  data_len is the .data file's length.
-DB_HD bool entry_readable(uint64_t offset, uint32_t full_size, uint64_t data_len) {
+DB_HOST_HD bool entry_readable(uint64_t offset, uint32_t full_size, uint64_t data_len) {
     return full_size != 0 && offset <= data_len && (uint64_t)full_size <= data_len - offset;
 }
 

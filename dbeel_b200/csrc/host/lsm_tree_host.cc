@@ -660,6 +660,156 @@ int dbeel_tree_scan_ranges(dbeel_tree *t, const dbeel_run *memtables, uint32_t n
     return rc;
 }
 
+// The file edge of a streamed scan (dbeel_scan_ranges_stream): the tables' descriptors (or the caller's memtables) on the
+// way in, two files per range on the way out, written like StreamFiles' outputs (mapped when the volume has room, else pwrite).
+namespace {
+struct ScanFiles {
+    std::vector<int> data_fd, index_fd;   // -1: a memtable, read from `mem`
+    std::vector<const dbeel_run *> mem;
+    std::vector<std::string> out_path;    // [2 r] = <r>.data, [2 r + 1] = <r>.index
+    std::vector<int> out_fd;
+    std::vector<uint8_t *> out_map;
+    std::vector<uint64_t> out_cap;
+    std::atomic<int> saved_errno{0};
+    void unmap() {
+        for (size_t k = 0; k < out_map.size(); k++)
+            if (out_map[k]) { munmap(out_map[k], out_cap[k]); out_map[k] = nullptr; }
+    }
+    ~ScanFiles() {
+        unmap();
+        for (int fd : data_fd) if (fd >= 0) close(fd);
+        for (int fd : index_fd) if (fd >= 0) close(fd);
+        for (int fd : out_fd) if (fd >= 0) close(fd);
+    }
+};
+
+int scan_read(void *ctx, uint32_t table, uint32_t kind, uint64_t off, uint64_t len, void *dst) {
+    auto *f = static_cast<ScanFiles *>(ctx);
+    if (table >= f->mem.size()) return DBEEL_ERR_INVALID_ARG;
+    if (const dbeel_run *m = f->mem[table]) {
+        const uint64_t n = kind == DBEEL_STREAM_DATA ? m->data_len : m->index_len;
+        if (off > n || len > n - off) return DBEEL_ERR_INVALID_ARG;
+        memcpy(dst, static_cast<const uint8_t *>(kind == DBEEL_STREAM_DATA ? m->data : m->index) + off, len);
+        return 0;
+    }
+    const int fd = kind == DBEEL_STREAM_DATA ? f->data_fd[table] : f->index_fd[table];
+    uint8_t *p = static_cast<uint8_t *>(dst);
+    while (len) {
+        const ssize_t r = pread(fd, p, len, (off_t)off);
+        if (r < 0 && errno == EINTR) continue;
+        if (r <= 0) { f->saved_errno.store(r < 0 ? errno : EIO); return DBEEL_ERR_IO; }
+        p += r; off += (uint64_t)r; len -= (uint64_t)r;
+    }
+    return 0;
+}
+
+int scan_write(void *ctx, uint32_t range, uint32_t kind, uint64_t off, const void *src, uint64_t len) {
+    auto *f = static_cast<ScanFiles *>(ctx);
+    if (kind != DBEEL_STREAM_DATA && kind != DBEEL_STREAM_INDEX) return DBEEL_ERR_INVALID_ARG;
+    const size_t k = 2ull * range + (kind == DBEEL_STREAM_INDEX ? 1 : 0);
+    if (k >= f->out_fd.size()) return DBEEL_ERR_INVALID_ARG;
+    if (f->out_map[k]) {
+        if (off > f->out_cap[k] || len > f->out_cap[k] - off) return DBEEL_ERR_CAPACITY;
+        memcpy(f->out_map[k] + off, src, len);
+        return 0;
+    }
+    const uint8_t *p = static_cast<const uint8_t *>(src);
+    while (len) {
+        const ssize_t r = pwrite(f->out_fd[k], p, len, (off_t)off);
+        if (r < 0 && errno == EINTR) continue;
+        if (r <= 0) { f->saved_errno.store(r < 0 ? errno : EIO); return DBEEL_ERR_IO; }
+        p += r; off += (uint64_t)r; len -= (uint64_t)r;
+    }
+    return 0;
+}
+} // namespace
+
+int dbeel_tree_scan_ranges_to_dir(dbeel_tree *t, const dbeel_run *memtables, uint32_t n_memtables, const dbeel_hash_range *ranges,
+                                  uint32_t n_ranges, uint32_t mode, const char *out_dir, dbeel_flush_table *per_range,
+                                  dbeel_scan_stop *stop) {
+    if (!t || (n_memtables && !memtables) || !stop || !out_dir || (n_ranges && !ranges)) return DBEEL_ERR_INVALID_ARG;
+    if (n_ranges > DBEEL_MAX_SCAN_RANGES) return DBEEL_ERR_INVALID_ARG;
+    t->err.clear();
+    // the same tables as dbeel_tree_scan_ranges: SSTables (ascending index), then the non-empty memtables
+    ScanFiles f;
+    std::vector<dbeel_run> tables;
+    std::vector<int32_t> position;
+    uint64_t in_data = 0, in_records = 0;
+    for (size_t i = 0; i < t->sstables.size(); i++) {
+        const std::string dp = file_path(t->dir, t->sstables[i].index, kData), ip = file_path(t->dir, t->sstables[i].index, kIndex);
+        const int dfd = open(dp.c_str(), O_RDONLY), ifd = open(ip.c_str(), O_RDONLY);
+        f.data_fd.push_back(dfd);
+        f.index_fd.push_back(ifd);
+        f.mem.push_back(nullptr);
+        struct stat sd, si;
+        if (dfd < 0 || ifd < 0 || fstat(dfd, &sd) != 0 || fstat(ifd, &si) != 0) return io_fail(t, "open " + dp);
+        tables.push_back(dbeel_run{nullptr, (uint64_t)sd.st_size, nullptr, (uint64_t)si.st_size});
+        position.push_back((int32_t)i);
+    }
+    for (uint32_t m = 0; m < n_memtables; m++) {
+        if (memtables[m].index_len < DBEEL_INDEX_ENTRY_SIZE) continue;
+        f.data_fd.push_back(-1);
+        f.index_fd.push_back(-1);
+        f.mem.push_back(&memtables[m]);
+        tables.push_back(memtables[m]);
+        position.push_back((int32_t)(t->sstables.size() + m));
+    }
+    for (const dbeel_run &r : tables) {
+        in_data += r.data_len;
+        in_records += r.index_len / DBEEL_INDEX_ENTRY_SIZE;
+    }
+    std::error_code ec;
+    fs::create_directories(out_dir, ec);
+    auto drop_outputs = [&]() { for (const std::string &p : f.out_path) unlink(p.c_str()); };
+    for (uint32_t r = 0; r < n_ranges; r++) {
+        for (const char *ext : {kData, kIndex}) {
+            const std::string p = (fs::path(out_dir) / (std::to_string(r) + "." + ext)).string();
+            const int fd = open(p.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644); // read-write: a shared writable mapping needs it
+            if (fd < 0) { const int rc = io_fail(t, "create " + p); drop_outputs(); return rc; }
+            f.out_path.push_back(p);
+            f.out_fd.push_back(fd);
+            f.out_map.push_back(nullptr);
+            f.out_cap.push_back(0);
+        }
+    }
+    if (stream_maps() && n_ranges) {
+        // Any one range can take every selected byte, so every file is mapped at the whole bound; the ranges are disjoint, so
+        // what they write together is the bound once: that is what the volume must have room for (see tree_compact_streamed).
+        const uint64_t cap_d = in_data, cap_i = 16 * in_records;
+        struct statvfs vfs;
+        if (fstatvfs(f.out_fd[0], &vfs) == 0 && (uint64_t)vfs.f_bavail * (uint64_t)vfs.f_frsize >= cap_d + cap_i + (64ull << 20)) {
+            for (size_t k = 0; k < f.out_fd.size(); k++) {
+                const uint64_t cap = k & 1 ? cap_i : cap_d;
+                if (!cap || ftruncate(f.out_fd[k], (off_t)cap) != 0) continue;
+                void *m = mmap(nullptr, cap, PROT_READ | PROT_WRITE, MAP_SHARED, f.out_fd[k], 0);
+                if (m == MAP_FAILED) { if (ftruncate(f.out_fd[k], 0) != 0) {} continue; }
+                f.out_map[k] = static_cast<uint8_t *>(m);
+                f.out_cap[k] = cap;
+            }
+        }
+    }
+    dbeel_scan_io io{scan_read, scan_write, &f};
+    int rc = dbeel_scan_ranges_stream(t->engine, tables.data(), (uint32_t)tables.size(), ranges, n_ranges, mode, &io, 0, per_range, stop);
+    if (stop->table >= 0 && (size_t)stop->table < position.size()) stop->table = position[stop->table];
+    if (rc) {
+        if (rc == DBEEL_ERR_IO) { errno = f.saved_errno.load(); io_fail(t, "streamed scan"); }
+        else t->err = dbeel_last_error(t->engine);
+        drop_outputs();
+        return rc;
+    }
+    f.unmap();
+    for (uint32_t r = 0; r < n_ranges; r++) {
+        for (int k = 0; k < 2; k++) { // cut to the final length (mapped files were sized to the bound)
+            const size_t j = 2ull * r + k;
+            const bool cut = ftruncate(f.out_fd[j], (off_t)(k ? per_range[r].index_len : per_range[r].data_len)) == 0;
+            const bool closed = close(f.out_fd[j]) == 0;
+            f.out_fd[j] = -1;
+            if (!cut || !closed) { rc = io_fail(t, "close " + f.out_path[j]); drop_outputs(); return rc; }
+        }
+    }
+    return DBEEL_OK;
+}
+
 int dbeel_tree_recover_wal(dbeel_tree *t, uint32_t tree_capacity, uint64_t *wal_file_index, uint64_t *items_written) {
     if (!t) return DBEEL_ERR_INVALID_ARG;
     t->err.clear();

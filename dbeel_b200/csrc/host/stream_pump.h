@@ -14,6 +14,11 @@
 //
 // so file reads, both PCIe directions and file writes all overlap, and the pinned memory is R slots however large the
 // SSTables are.  Any callback error aborts the pump; the first error code is what every wait returns from then on.
+//
+// A partition's output is either one .data and one .index piece of a single output (publish_out, the compaction) or any
+// number of pieces that each name an output stream, a kind and an offset (publish_pieces, the streamed scan: one output
+// stream per hash range, written through the stream-write callback).  end_at(n) ends the walk after partition n - 1: the
+// later partitions are never read, published or written (the scan stops there).
 #pragma once
 #include <stdint.h>
 
@@ -42,6 +47,13 @@ class StreamPump {
         const uint8_t *index = nullptr;
         uint64_t index_len = 0, index_off = 0;
     };
+    struct OutPiece { // one piece of a multi-stream partition: len bytes at src go to offset `off` of (stream, kind)
+        const uint8_t *src = nullptr;
+        uint64_t len = 0;
+        uint32_t stream = 0, kind = 0;
+        uint64_t off = 0;
+    };
+    typedef int (*StreamWriteFn)(void *ctx, uint32_t stream, uint32_t kind, uint64_t offset, const void *src, uint64_t len);
     static constexpr uint64_t kPiece = 8ull << 20; // bytes per callback call
 
     // wait_out(c): blocks until partition c's output has arrived in host memory (the engine: cudaEventSynchronize).
@@ -50,7 +62,7 @@ class StreamPump {
                std::function<void()> thread_init = nullptr)
         : io_(io), np_(n_parts), ring_(ring ? ring : 1), nt_(n_threads > 0 ? n_threads : 1), wait_out_(std::move(wait_out)),
           thread_init_(std::move(thread_init)), r_left_(n_parts, 0), w_left_(n_parts, 0), w_next_(new std::atomic<uint64_t>[n_parts ? n_parts : 1]),
-          outs_(n_parts) {
+          chunks_(n_parts), end_(n_parts) {
         for (uint32_t c = 0; c < n_parts; c++) w_next_[c].store(0);
     }
     StreamPump(const StreamPump &) = delete;
@@ -68,6 +80,9 @@ class StreamPump {
             r_left_[part]++;
         }
     }
+
+    // Before start(): the callback publish_pieces writes through (ctx = the read callback's).
+    void set_stream_write(StreamWriteFn fn) { stream_write_ = fn; }
 
     void start() {
         started_ = true;
@@ -97,10 +112,22 @@ class StreamPump {
     }
 
     void publish_out(uint32_t part, const OutPart &o) {
+        std::vector<Chunk> ch;
+        split(&ch, o.data, o.data_len, 0, DBEEL_STREAM_DATA, o.data_off, false);
+        split(&ch, o.index, o.index_len, 0, DBEEL_STREAM_INDEX, o.index_off, false);
+        publish(part, std::move(ch));
+    }
+
+    void publish_pieces(uint32_t part, const std::vector<OutPiece> &ps) {
+        std::vector<Chunk> ch;
+        for (const OutPiece &q : ps) split(&ch, q.src, q.len, q.stream, q.kind, q.off, true);
+        publish(part, std::move(ch));
+    }
+
+    // Partitions [n, n_parts) will not be published: their reads are skipped and finish() does not wait for them.
+    void end_at(uint32_t n) {
         std::lock_guard<std::mutex> lk(mu_);
-        outs_[part] = o;
-        w_left_[part] = pieces(o.data_len) + pieces(o.index_len);
-        published_ = part + 1;
+        if (n < end_) end_ = n;
         cv_.notify_all();
     }
 
@@ -110,8 +137,8 @@ class StreamPump {
             std::unique_lock<std::mutex> lk(mu_);
             cv_.wait(lk, [&] {
                 if (failed_) return true;
-                if (published_ < np_) return false;
-                for (uint32_t c = 0; c < np_; c++)
+                if (published_ < end_) return false;
+                for (uint32_t c = 0; c < end_; c++)
                     if (w_left_[c]) return false;
                 return true;
             });
@@ -132,7 +159,26 @@ class StreamPump {
     }
 
   private:
-    static uint64_t pieces(uint64_t len) { return (len + kPiece - 1) / kPiece; }
+    struct Chunk { // one write callback call
+        const uint8_t *src;
+        uint64_t len;
+        uint32_t stream, kind;
+        uint64_t off;
+        bool multi; // through stream_write_
+    };
+
+    static void split(std::vector<Chunk> *ch, const uint8_t *src, uint64_t len, uint32_t stream, uint32_t kind, uint64_t off, bool multi) {
+        for (uint64_t done = 0; done < len; done += kPiece)
+            ch->push_back(Chunk{src + done, len - done < kPiece ? len - done : kPiece, stream, kind, off + done, multi});
+    }
+
+    void publish(uint32_t part, std::vector<Chunk> ch) {
+        std::lock_guard<std::mutex> lk(mu_);
+        chunks_[part] = std::move(ch);
+        w_left_[part] = chunks_[part].size();
+        published_ = part + 1;
+        cv_.notify_all();
+    }
 
     void join() {
         for (auto &t : threads_)
@@ -155,8 +201,9 @@ class StreamPump {
             const ReadTask &t = tasks_[k];
             {
                 std::unique_lock<std::mutex> lk(mu_);
-                cv_.wait(lk, [&] { return failed_ || t.part < consumed_ + ring_; });
+                cv_.wait(lk, [&] { return failed_ || t.part >= end_ || t.part < consumed_ + ring_; });
                 if (failed_) return;
+                if (t.part >= end_) continue;
             }
             const int rc = io_->read(io_->ctx, t.run, t.kind, t.off, t.len, t.dst);
             std::lock_guard<std::mutex> lk(mu_);
@@ -170,24 +217,21 @@ class StreamPump {
     void writer() {
         if (thread_init_) thread_init_();
         for (uint32_t c = 0; c < np_; c++) {
-            OutPart o;
             {
                 std::unique_lock<std::mutex> lk(mu_);
-                cv_.wait(lk, [&] { return failed_ || published_ > c; });
-                if (failed_) return;
-                o = outs_[c];
+                cv_.wait(lk, [&] { return failed_ || c >= end_ || published_ > c; });
+                if (failed_ || c >= end_) return;
             }
-            const uint64_t nd = pieces(o.data_len), total = nd + pieces(o.index_len);
+            const std::vector<Chunk> &ch = chunks_[c]; // not modified once published
+            const uint64_t total = ch.size();
             if (total == 0) continue;
             if (wait_out_) wait_out_(c);
             while (true) {
                 const uint64_t k = w_next_[c].fetch_add(1);
                 if (k >= total) break;
-                const bool is_data = k < nd;
-                const uint64_t q = is_data ? k : k - nd, len_all = is_data ? o.data_len : o.index_len;
-                const uint64_t off = q * kPiece, n = len_all - off < kPiece ? len_all - off : kPiece;
-                const int rc = io_->write(io_->ctx, is_data ? DBEEL_STREAM_DATA : DBEEL_STREAM_INDEX, (is_data ? o.data_off : o.index_off) + off,
-                                          (is_data ? o.data : o.index) + off, n);
+                const Chunk &q = ch[k];
+                const int rc = q.multi ? stream_write_(io_->ctx, q.stream, q.kind, q.off, q.src, q.len)
+                                       : io_->write(io_->ctx, q.kind, q.off, q.src, q.len);
                 std::lock_guard<std::mutex> lk(mu_);
                 if (rc) fail_locked(rc);
                 w_left_[c]--;
@@ -210,7 +254,9 @@ class StreamPump {
     std::vector<uint32_t> r_left_;
     std::vector<uint64_t> w_left_;
     std::unique_ptr<std::atomic<uint64_t>[]> w_next_;
-    std::vector<OutPart> outs_;
+    std::vector<std::vector<Chunk>> chunks_;
+    StreamWriteFn stream_write_ = nullptr;
+    uint32_t end_;           // partitions [end_, np_) are skipped
     uint32_t consumed_ = 0;  // partitions [0, consumed_) have released their input slot
     uint32_t published_ = 0; // partitions [0, published_) have their output described
     bool failed_ = false, done_ = false, started_ = false;

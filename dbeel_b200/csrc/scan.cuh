@@ -18,6 +18,15 @@
 //   k_scan_res_tiles  per 128 res records: bytes and entries (what k_resolve leaves for the offsets scan)
 //   k_scan_tiles, k_scan_chunks, k_emit, k_gather32 / k_gather, k_flush_table, k_rebase_index
 //                     exactly as a flush-many job runs them: every range's output is one file-relative SSTable
+//
+// The streamed form (dbeel_scan_ranges_stream) runs the same sequence once per partition (host/scan_plan.h: a run of
+// consecutive records whose .data spans and index slices sit in a ring slot), with partition-local ordinals.  What
+// crosses partitions stays on the device, so no partition waits for the host to learn about the one before it:
+//
+//   k_scan_part_enter      the partition's stop word: 0 (keep nothing) when an earlier partition stopped the scan
+//   k_scan_rebase_stream   instead of k_rebase_index: .index offsets relative to the start of the range's whole stream
+//   k_scan_part_leave      fold the partition's stop into the global one, add its per-range (bytes, items) to the running
+//                          totals, write every range's piece (place in the output, stream offsets) to the pinned header
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -141,6 +150,67 @@ __global__ void __launch_bounds__(kResolveThreads) k_scan_res_tiles(Params p, co
         p.tile_bytes[blockIdx.x] = b;
         p.tile_count[blockIdx.x] = c;
     }
+}
+
+// ---- the streamed scan's cross-partition state
+
+// One thread.  global_stop: (global ordinal << 2) | reason of the record that stopped the scan, ~0 = none yet.
+__global__ void k_scan_part_enter(unsigned long long *local_stop, const unsigned long long *global_stop) {
+    *local_stop = *global_stop == ~0ull ? ~0ull : 0ull; // 0: k_route_hash<true> drops every record of this partition
+}
+
+// k_rebase_index for a partition of a streamed scan: the offsets k_emit wrote count from the partition's output start;
+// every range's stream continues where the range's pieces of the earlier partitions ended (run_tot[2 r], before
+// k_scan_part_leave adds this partition).
+__global__ void __launch_bounds__(256) k_scan_rebase_stream(Params p, const unsigned long long *run_tot) {
+    const uint32_t e = blockIdx.x * 256u + threadIdx.x;
+    if (e >= p.ctl->out_items) return;
+    uint32_t lo = 0, hi = p.n_groups; // last range whose first entry is <= e (empty ranges share a boundary)
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (p.mem_table[2 * mid + 1] <= e) lo = mid; else hi = mid;
+    }
+    uint4 rec = p.out_index[e];
+    const unsigned long long off = ((unsigned long long)rec.x | ((unsigned long long)rec.y << 32)) - p.mem_table[2 * lo] + run_tot[2 * lo];
+    rec.x = (uint32_t)off;
+    rec.y = (uint32_t)(off >> 32);
+    p.out_index[e] = rec;
+}
+
+// The per-range row of the pinned header (host/device mapped) that k_scan_part_leave writes for every partition.
+struct ScanPieceRow {
+    unsigned long long data_at, data_len; // .data bytes [data_at, data_at + data_len) of the partition's output
+    unsigned long long items;             // .index records [items_at, items_at + items) of it
+    unsigned long long items_at;
+    unsigned long long stream_data_off, stream_items_off; // where they go in the range's stream (.index: 16 x items_off)
+};
+
+// One CTA.  mem_table: k_flush_table's rows of the partition; run_tot[2 r] / [2 r + 1]: .data bytes / items of range r
+// written by the earlier partitions.  hdr: the global stop word, then n_ranges rows.
+__global__ void k_scan_part_leave(const unsigned long long *mem_table, uint32_t n_ranges, const unsigned long long *local_stop,
+                                  unsigned long long *global_stop, unsigned long long first_ordinal, unsigned long long *run_tot,
+                                  unsigned long long *hdr) {
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const unsigned long long l = *local_stop;
+        if (*global_stop == ~0ull && l != ~0ull) *global_stop = ((first_ordinal + (l >> 2)) << 2) | (l & 3);
+        hdr[0] = *global_stop;
+    }
+    ScanPieceRow *rows = reinterpret_cast<ScanPieceRow *>(hdr + 1);
+    for (uint32_t r = threadIdx.x; r < n_ranges; r += blockDim.x) {
+        const unsigned long long b0 = mem_table[2 * r], b1 = mem_table[2 * (r + 1)], i0 = mem_table[2 * r + 1], i1 = mem_table[2 * (r + 1) + 1];
+        ScanPieceRow row;
+        row.data_at = b0;
+        row.data_len = b1 - b0;
+        row.items_at = i0;
+        row.items = i1 - i0;
+        row.stream_data_off = run_tot[2 * r];
+        row.stream_items_off = run_tot[2 * r + 1];
+        rows[r] = row;
+        run_tot[2 * r] += b1 - b0;
+        run_tot[2 * r + 1] += i1 - i0;
+    }
+    __threadfence_system(); // visible to the host before the stream reports completion
 }
 
 } // namespace dbeel

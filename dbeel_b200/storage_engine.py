@@ -9,6 +9,7 @@ All the work happens in the C++/CUDA library; this file only marshals arguments.
 from __future__ import annotations
 
 import ctypes as C
+import os
 from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -51,6 +52,9 @@ def _lib():
         L.dbeel_tree_scan_ranges.restype = C.c_int
         L.dbeel_tree_scan_ranges.argtypes = [C.c_void_p, C.POINTER(capi.Run), C.c_uint32, C.POINTER(capi.HashRange), C.c_uint32,
                                              C.c_uint32, C.POINTER(capi.Out), C.POINTER(capi.FlushTable), C.POINTER(capi.ScanStop)]
+        L.dbeel_tree_scan_ranges_to_dir.restype = C.c_int
+        L.dbeel_tree_scan_ranges_to_dir.argtypes = [C.c_void_p, C.POINTER(capi.Run), C.c_uint32, C.POINTER(capi.HashRange), C.c_uint32,
+                                                    C.c_uint32, C.c_char_p, C.POINTER(capi.FlushTable), C.POINTER(capi.ScanStop)]
         L.dbeel_tree_recover_wal.restype = C.c_int
         L.dbeel_tree_recover_wal.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.dbeel_tree_last_error.restype = C.c_char_p
@@ -70,7 +74,7 @@ def _lib():
 
 
 TREE_EXPORTS = ["dbeel_tree_open", "dbeel_tree_close", "dbeel_tree_sstables", "dbeel_tree_write_sstable_index",
-                "dbeel_tree_compact", "dbeel_tree_compact_many", "dbeel_tree_flush", "dbeel_tree_recover_wal", "dbeel_tree_get_many", "dbeel_tree_scan_ranges", "dbeel_tree_last_error", "dbeel_memtable_cut",
+                "dbeel_tree_compact", "dbeel_tree_compact_many", "dbeel_tree_flush", "dbeel_tree_recover_wal", "dbeel_tree_get_many", "dbeel_tree_scan_ranges", "dbeel_tree_scan_ranges_to_dir", "dbeel_tree_last_error", "dbeel_memtable_cut",
                 "dbeel_plan_compactions", "dbeel_out_pages", "dbeel_tree_set_page_sink"]
 
 
@@ -211,6 +215,20 @@ class LSMTree:
                                                   C.byref(stop)), "LSMTree.scan_ranges")
         rows, st = capi.Engine._scan_result(per_range, len(ranges), stop)
         return od[:out.data_len], oi[:out.index_len], rows, st
+
+    def scan_ranges_to_dir(self, ranges: Sequence[Tuple[int, int]], out_dir: str, mode: int = capi.SCAN_REFERENCE,
+                           memtables=()):
+        """scan_ranges streamed from the tree's files: range r goes to <out_dir>/<r>.data and <out_dir>/<r>.index
+        (dbeel_tree_scan_ranges_to_dir).  Returns (per_range, stop): per_range rows with data_off == index_off == 0, stop
+        as in scan_ranges."""
+        keep = [(capi._u8(d), capi._u8(i)) for d, i in memtables]
+        mts = (capi.Run * max(1, len(keep)))()
+        for j, (d, i) in enumerate(keep):
+            mts[j] = capi.Run(d.ctypes.data, d.size, i.ctypes.data, i.size)
+        rng, per_range, stop = capi.Engine._scan_args(ranges)
+        self._check(_lib().dbeel_tree_scan_ranges_to_dir(self._h, mts, len(keep), rng, len(ranges), mode, os.fsencode(out_dir),
+                                                         per_range, C.byref(stop)), "LSMTree.scan_ranges_to_dir")
+        return capi.Engine._scan_result(per_range, len(ranges), stop)
 
     def recover_wal(self, tree_capacity: int = capi.DEFAULT_TREE_CAPACITY) -> Tuple[int, int]:
         """open_or_create_ex's WAL step (lsm_tree.rs:466-513): with two `.memtable` files the older one is replayed and

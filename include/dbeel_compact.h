@@ -397,6 +397,36 @@ int dbeel_scan_ranges_device(dbeel_engine *e, const dbeel_run *tables, uint32_t 
                              uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range,
                              dbeel_scan_stop *stop);
 
+/* The same scan fed from files, one output stream per range (shard migration sends every range's entries to another
+ * shard, over a socket or a channel).  The engine moves the bytes
+ *     file -> read() -> pinned ring -> H2D -> kernels -> D2H -> pinned ring -> write(range) -> the range's stream
+ * one partition at a time, so the page-locked and device memory is a few partitions however large the tree is.  A
+ * partition is a run of consecutive records in iteration order (it may span tables) whose index slices and .data spans
+ * take at most partition_bytes (0 = the engine's partition size); a single record larger than that gets a partition of
+ * its own.  tables[i].data / .index are ignored (lengths only); every table's .index is read whole first (16 bytes per
+ * record), the .data files partition by partition.
+ *   read : fill dst with [offset, offset + len) of table `table`'s .data (DBEEL_STREAM_DATA) or .index (DBEEL_STREAM_INDEX)
+ *   write: store len bytes at `offset` of range `range`'s .data (DBEEL_STREAM_DATA) or .index (DBEEL_STREAM_INDEX) stream
+ * Both are called from several engine threads at once and return 0 or an error code of the caller's, which
+ * dbeel_scan_ranges_stream returns unchanged; the engine stays usable after one.  Pieces arrive in no particular order;
+ * a range that selects nothing gets no write call.
+ *
+ * Range r's stream is byte for byte what dbeel_scan_ranges puts at per_range[r] for the same tables, ranges and mode: its
+ * .data bytes, and its .index records with offsets relative to the range's own .data.  per_range[r] has data_off ==
+ * index_off == 0 (every range is its own stream) and the lengths and items of dbeel_scan_ranges.  *stop is the same, and
+ * nothing after the stop is ever written.  There is no output capacity (no DBEEL_ERR_CAPACITY).  The 2^32-record limit
+ * of dbeel_scan_ranges applies per partition, not per call.  dbeel_last_stats fills partitions (partitions scanned), the
+ * entries_* counts, input_bytes and output_bytes; ms_h2d, ms_total and ms_d2h are the sums over the partitions of the
+ * H2D copies, the kernels and the D2H copies (they overlap each other and the callbacks). */
+typedef struct dbeel_scan_io {
+    int (*read)(void *ctx, uint32_t table, uint32_t kind, uint64_t offset, uint64_t len, void *dst);
+    int (*write)(void *ctx, uint32_t range, uint32_t kind, uint64_t offset, const void *src, uint64_t len);
+    void *ctx;
+} dbeel_scan_io;
+int dbeel_scan_ranges_stream(dbeel_engine *e, const dbeel_run *tables, uint32_t n_tables, const dbeel_hash_range *ranges,
+                             uint32_t n_ranges, uint32_t mode, const dbeel_scan_io *io, uint64_t partition_bytes,
+                             dbeel_flush_table *per_range, dbeel_scan_stop *stop);
+
 /* Bloom::new_for_fp_rate arithmetic (bloomfilter 1.0.12). */
 uint64_t dbeel_bloom_bitmap_bytes(uint64_t items, double fp);
 uint32_t dbeel_bloom_k_num(uint64_t bitmap_bits, uint64_t items);

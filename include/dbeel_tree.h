@@ -19,6 +19,8 @@
  *   dbeel_tree_get_many    <- the SSTable loop of LSMTree::get_entry (lsm_tree.rs:686-719) through dbeel_get_many()
  *   dbeel_tree_scan_ranges <- migrate_actions' scan over iter_filter (src/tasks/migration.rs:62-131) through
  *                             dbeel_scan_ranges()
+ *   dbeel_tree_scan_ranges_to_dir <- the same scan streamed from the tree's files through dbeel_scan_ranges_stream(),
+ *                             one pair of files per range
  *   dbeel_memtable_cut     <- RedBlackTree::set + active_memtable_full (rbtree_arena lib.rs:497-534,
  *                             lsm_tree.rs:600-603,757-765): how many arrivals fill one memtable
  *   dbeel_plan_compactions <- compact_tree's size-tiered picker (src/tasks/compaction.rs:35-102),
@@ -85,6 +87,16 @@ int dbeel_tree_get_many(dbeel_tree *t, const void *keys, const uint64_t *key_off
 int dbeel_tree_scan_ranges(dbeel_tree *t, const dbeel_run *memtables, uint32_t n_memtables, const dbeel_hash_range *ranges,
                            uint32_t n_ranges, uint32_t mode, dbeel_out *out, dbeel_flush_table *per_range,
                            dbeel_scan_stop *stop);
+
+/* The same scan, streamed: the SSTables are read from their files with pread, partition by partition, the memtables from
+ * the caller's memory, through dbeel_scan_ranges_stream() (the tree's files are never held whole in memory).  Range r goes
+ * to <out_dir>/<r>.data and <out_dir>/<r>.index (out_dir is created if missing): the bytes of range r's slice of
+ * dbeel_tree_scan_ranges, its .index offsets relative to <r>.data.  Every file is cut to its final length; a range that
+ * selects nothing leaves two empty files.  per_range rows have data_off == index_off == 0; stop as in
+ * dbeel_tree_scan_ranges.  On an error every file this call created is removed. */
+int dbeel_tree_scan_ranges_to_dir(dbeel_tree *t, const dbeel_run *memtables, uint32_t n_memtables, const dbeel_hash_range *ranges,
+                                  uint32_t n_ranges, uint32_t mode, const char *out_dir, dbeel_flush_table *per_range,
+                                  dbeel_scan_stop *stop);
 
 /* WAL recovery step of open_or_create_ex.  0 logs: *wal_file_index = 0; 1 log: its index; 2 logs: the older one is
  * replayed (memtable of `tree_capacity` entries, DBEEL_ERR_TREE_FULL like the reference's ReachedCapacity), flushed
